@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- columns/s of the SB+ML+MU CAPE/CIN/LCL/LFC/EL suite on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the fused suite kernel over this rank's column block.  The default
@@ -18,6 +18,13 @@ with HOST buffers (pinned host -> device -> kernel -> host inside the timed regi
 ``roofline`` = algorithmic bytes / kernel time against MEASURED_PEAKS.json; ``cpu_baseline`` =
 the NumPy oracle (restated reference) timed on this box's host cores on a bounded sample.
 ``--impl reference`` times that CPU restatement alone, with all host cores.
+
+``--dump-outputs DIR`` writes the arrays the last timed step returned, one ``DIR/<kind>_<field>.npy`` per output, so
+that two builds can be compared output for output (the inputs are seeded: the same arguments give the same inputs).
+Undefined outputs (NaN: no LFC / EL) are written as 0 beside a ``DIR/<kind>_<field>_defined.npy`` mask, so every
+file is finite.  Outputs larger than 60 MB in all are cut to the same seeded sample of columns in every file.
+
+The tree is only read (it may be read-only): no bytecode is written and the oracle's tables are regenerated in memory.
 """
 
 import argparse
@@ -58,7 +65,14 @@ def parse_args():
     ap.add_argument("--ref-columns", type=int, default=0, help="--impl reference: columns per step")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the extra lines of the default run (other BASELINE configs, float64 I/O, pageable e2e)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<kind>_<field>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
+    return args
 
 
 # ------------------------------------------------------------------------------- workloads
@@ -187,7 +201,7 @@ def oracle_setup(kinds):
     global _ORACLE_TABLES, _ORACLE_KINDS
     from oracle import tables as otab
     if _ORACLE_TABLES is None:
-        _ORACLE_TABLES = otab.load_tables()      # regenerated (~10 s) when oracle/_cache is absent
+        _ORACLE_TABLES = otab.load_tables(cache=False)      # ~10 s; no cache file in the tree
     _ORACLE_KINDS = tuple(kinds)
 
 
@@ -322,6 +336,8 @@ def run_b200(args):
         evs[i + 1].record()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:          # before later loops reuse `outs`
+        dump_outputs(args.dump_outputs, outs, spec["N"])
     total_ms = evs[0].elapsed_time(evs[-1])
     per_ms = sorted(evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps))
     kernel_ms = sum(per_ms) / len(per_ms)
@@ -436,6 +452,42 @@ def run_b200(args):
         dist.destroy_process_group()
 
 
+DUMP_BYTES = 60_000_000       # --dump-outputs: under 64 MB with the .npy headers
+DUMP_SEED = 20261020
+
+
+def dump_outputs(out_dir, outs, n_columns):
+    """Write every output block of ``ctx.alloc_outputs`` as out_dir/<kind>_<field>.npy ([N] scalars, [L+1, N]
+    profile rows).  An output the library leaves undefined is NaN (no LFC / EL, all-NaN input column); the dump keeps
+    every file finite: such entries are written as 0 and <kind>_<field>_defined.npy holds 1 where the value is
+    defined and 0 where it is not (one for every output, so the file set does not depend on the data).  When the
+    whole set exceeds DUMP_BYTES, every file holds the same sorted sample of columns drawn with DUMP_SEED, so dumps
+    of two builds with the same arguments line up column for column."""
+    import numpy as np
+    import torch
+    from xarray_parcel_b200._lib import PROFILE_FIELDS
+    arrays = {}
+    for kind, (_, scal, _, prof, names) in outs.items():
+        for i, f in enumerate(names):
+            arrays[f"{kind}_{f}"] = scal[i]
+        if prof is not None:
+            for i, f in enumerate(PROFILE_FIELDS):
+                arrays[f"{kind}_{f}"] = prof[i]
+    per_column = 2 * sum(a.numel() // n_columns * a.element_size() for a in arrays.values())    # values + masks
+    n = min(n_columns, DUMP_BYTES // per_column)
+    idx = None
+    if n < n_columns:
+        pick = np.sort(np.random.default_rng(DUMP_SEED).choice(n_columns, n, replace=False))
+        idx = torch.from_numpy(pick).to(next(iter(arrays.values())).device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if idx is not None:
+            a = a.index_select(a.dim() - 1, idx)
+        defined = torch.isfinite(a)
+        np.save(os.path.join(out_dir, name + ".npy"), torch.where(defined, a, torch.zeros_like(a)).cpu().numpy())
+        np.save(os.path.join(out_dir, name + "_defined.npy"), defined.to(a.dtype).cpu().numpy())
+
+
 def _time_device(fn, steps, warmup):
     import torch
     for _ in range(warmup):
@@ -538,6 +590,7 @@ def _emit(line):
 
 
 def main():
+    sys.dont_write_bytecode = True
     _claim_stdout()
     args = parse_args()
     if args.impl == "reference":
