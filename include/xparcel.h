@@ -334,6 +334,26 @@ xp_status xp_virtual_temperature(xp_context *ctx, const void *temperature, const
  * (PF:525-607, lookup tables) from the LCL back to the point's pressure.  Needs the tables. */
 xp_status xp_wet_bulb_temperature(xp_context *ctx, const void *pressure, const void *temperature,
                                   const void *dewpoint, int64_t n, int32_t dtype, void *wet_bulb, void *stream);
+/* xp_downdraft_cape: downdraft CAPE (MetPy's downdraft_cape recipe) per column, device memory only.
+ * Contract (DESIGN.md section 3.12): a level is valid when p, T and Td are non-NaN; the downdraft starts at the point
+ * of minimum equivalent potential temperature (Bolton) among the valid levels in 700-500 hPa (np.isclose to a bound
+ * counts as inside) and the points at exactly 700 / 500 hPa interpolated in ln p where no level is close to a bound
+ * (first minimum, the larger pressure, on a tie); the start temperature is the Normand wet bulb there; the parcel
+ * descends on the table adiabat nearest to (start pressure, wet bulb) to every valid level at or below the start;
+ * dcape = -Rd * trapezoid(Tv_env - Tv_parcel, ln p) from the surface up, in J/kg, not clipped (negative where the
+ * parcel is warmer).  A column that cannot bracket 700 and 500 hPa, a NaN theta-e or a table index of 0 gives NaN in
+ * every output.  metpy_compat (141 / 162) selects the environment's mixing ratio form as in xp_mixing_ratio.
+ * Outputs: dcape [J/kg], start_pressure [hPa], start_temperature [K] ([n_columns] each) and parcel_temperature
+ * ([n_levels][n_columns] with level stride parcel_level_stride: the descending parcel, NaN above the start and on
+ * invalid levels); a NULL output is skipped.  Needs the tables (XP_ERR_TABLES_NOT_LOADED). */
+typedef struct xp_downdraft_out {
+    void *dcape, *start_pressure, *start_temperature, *parcel_temperature;
+    int64_t parcel_level_stride;
+} xp_downdraft_out;
+xp_status xp_downdraft_cape(xp_context *ctx, const void *pressure, int64_t pressure_level_stride,
+                            int32_t pressure_is_1d, const void *temperature, const void *dewpoint,
+                            int64_t level_stride, int32_t n_levels, int64_t n_columns, int32_t dtype,
+                            int32_t metpy_compat, const xp_downdraft_out *out, void *stream);
 /* significant_hail_parameter (PF:2261-2306): units as the reference's arguments (mixing ratio kg/kg,
  * lapse K/km negative for decreasing temperature, temp_500 K, shear m/s, flh m). */
 xp_status xp_significant_hail_parameter(xp_context *ctx, const void *mucape, const void *mixing_ratio,

@@ -66,7 +66,7 @@ EXPORTS = ["xp_version", "xp_create", "xp_destroy", "xp_last_error", "xp_take_fl
            "xp_dry_lapse", "xp_mixing_ratio", "xp_virtual_temperature", "xp_wet_bulb_temperature",
            "xp_significant_hail_parameter", "xp_storm_proxies", "xp_mixed_layer", "xp_mixed_parcel",
            "xp_layer_bounds", "xp_insert_level", "xp_shift_out_nans", "xp_trapz", "xp_valid_data",
-           "xp_find_intersections", "xp_interp1d", "xp_trap_around_zeros"]
+           "xp_find_intersections", "xp_interp1d", "xp_trap_around_zeros", "xp_downdraft_cape"]
 
 PROXY_INPUTS = ["mixed_100_cape", "mixed_50_cape", "mu_cape", "shear_magnitude", "mixed_100_lifted_index",
                 "mixed_100_dci", "positive_shear", "mixed_50_cin", "mixed_100_cin", "lapse_rate_700_500",
@@ -95,6 +95,14 @@ ZERO_AREA_FIELDS = ["area", "x", "dx", "x_from", "x_to"]
 
 class XpZeroAreasOut(ctypes.Structure):
     _fields_ = [(n, c_void_p) for n in ZERO_AREA_FIELDS] + [("mask", c_void_p)]
+
+
+DOWNDRAFT_FIELDS = ["dcape", "downdraft_start_pressure", "downdraft_start_temperature"]
+
+
+class XpDowndraftOut(ctypes.Structure):
+    _fields_ = [("dcape", c_void_p), ("start_pressure", c_void_p), ("start_temperature", c_void_p),
+                ("parcel_temperature", c_void_p), ("parcel_level_stride", c_int64)]
 
 
 class XpProxyInputs(ctypes.Structure):
@@ -198,6 +206,8 @@ def load_library():
                                     c_int32, c_void_p]
         lib.xp_trap_around_zeros.argtypes = [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_int64, c_int64, c_int32,
                                              c_int64, c_int32, c_int32, ctypes.POINTER(XpZeroAreasOut), c_void_p]
+        lib.xp_downdraft_cape.argtypes = [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_int64, c_int32,
+                                          c_int64, c_int32, c_int32, ctypes.POINTER(XpDowndraftOut), c_void_p]
         lib.xp_launch_count.argtypes = [c_void_p]
         lib.xp_launch_count.restype = ctypes.c_uint64
         lib.xp_last_kernel_ms.argtypes = [c_void_p, ctypes.POINTER(ctypes.c_float)]
@@ -593,6 +603,37 @@ class Context:
                                       bottom.data_ptr(), top.data_ptr(), self._stream())
         self._check(st, "xp_layer_bounds")
         return bottom, top
+
+    def downdraft_cape(self, pressure, temperature, dewpoint, metpy_compat="1.4.1", profile=False, outputs=None):
+        """Downdraft CAPE (xp_downdraft_cape) of the columns of ``temperature`` / ``dewpoint`` [L, N] on ``pressure``
+        ([L, N] or a shared [L]; any level stride).  Returns a dict of the DOWNDRAFT_FIELDS [N] and, with
+        ``profile``, 'downdraft_parcel_temperature' [L, N].  ``outputs`` (a subset of those names) leaves the others
+        uncomputed (NULL in the call)."""
+        compat = {"1.4.1": 141, "1.6.2": 162, 141: 141, 162: 162, "141": 141, "162": 162}[metpy_compat]
+        L, N = temperature.shape
+        dt = temperature.dtype
+        dewpoint = dewpoint.to(dt)
+        if not (temperature.stride(1) == 1 and dewpoint.stride(1) == 1 and temperature.stride(0) == dewpoint.stride(0)):
+            temperature, dewpoint = temperature.contiguous(), dewpoint.contiguous()
+        pressure = pressure.to(dt)
+        p1d = pressure.dim() == 1
+        if not p1d and pressure.stride(1) != 1:
+            pressure = pressure.contiguous()
+        names = list(DOWNDRAFT_FIELDS) + (["downdraft_parcel_temperature"] if profile else [])
+        if outputs is not None:
+            names = [n for n in names if n in outputs]
+        dev = temperature.device
+        res = {n: torch.empty((L, N) if n == "downdraft_parcel_temperature" else (N,), dtype=dt, device=dev)
+               for n in names}
+        ptr = {n: res[n].data_ptr() if n in res else None
+               for n in DOWNDRAFT_FIELDS + ["downdraft_parcel_temperature"]}
+        o = XpDowndraftOut(ptr["dcape"], ptr["downdraft_start_pressure"], ptr["downdraft_start_temperature"],
+                           ptr["downdraft_parcel_temperature"], N)
+        st = self.lib.xp_downdraft_cape(self.handle, pressure.data_ptr(), pressure.stride(0), int(p1d),
+                                        temperature.data_ptr(), dewpoint.data_ptr(), temperature.stride(0), L, N,
+                                        _dtype_code(temperature), compat, ctypes.byref(o), self._stream())
+        self._check(st, "xp_downdraft_cape")
+        return res
     # ---- level primitives (xp_levels.cu) ---------------------------------------------------------------
     @staticmethod
     def _ptrs(tensors):

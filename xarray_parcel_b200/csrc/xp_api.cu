@@ -1104,6 +1104,33 @@ xp_status xp_wet_bulb_temperature(xp_context *ctx, const void *pressure, const v
     return check_cuda(ctx, cudaGetLastError(), "wet_bulb_temperature kernel launch");
 }
 
+// Downdraft CAPE, contract in include/xparcel.h and xp_downdraft.cuh (DESIGN.md section 3.12).
+xp_status xp_downdraft_cape(xp_context *ctx, const void *pressure, int64_t pressure_level_stride,
+                            int32_t pressure_is_1d, const void *temperature, const void *dewpoint,
+                            int64_t level_stride, int32_t n_levels, int64_t n_columns, int32_t dtype,
+                            int32_t metpy_compat, const xp_downdraft_out *out, void *stream) {
+    if (!ctx) return XP_ERR_INVALID_ARGUMENT;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if (!ctx->tables) return fail(ctx, XP_ERR_TABLES_NOT_LOADED, "Call load_moist_adiabat_lookups first.");
+    if (n_columns == 0) return XP_OK;
+    if (!pressure || !temperature || !dewpoint || !out || n_levels < 1 || n_columns < 0 ||
+        (metpy_compat != 141 && metpy_compat != 162))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad downdraft_cape arguments");
+    if (n_levels > 1 && (level_stride < n_columns ||
+                         pressure_level_stride < (pressure_is_1d ? 1 : n_columns) ||
+                         (out->parcel_temperature && out->parcel_level_stride < n_columns)))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "downdraft_cape: level strides smaller than a level");
+    if (!out->dcape && !out->start_pressure && !out->start_temperature && !out->parcel_temperature) return XP_OK;
+    DeviceGuard guard(ctx->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    const Tables tb = {ctx->d_index, ctx->d_curves};
+    XP_DISPATCH(dtype,
+                launch_downdraft_cape<float>((const float *)pressure, pressure_level_stride, pressure_is_1d, (const float *)temperature, (const float *)dewpoint, level_stride, n_levels, n_columns, metpy_compat, tb, (float *)out->dcape, (float *)out->start_pressure, (float *)out->start_temperature, (float *)out->parcel_temperature, out->parcel_level_stride, st),
+                launch_downdraft_cape<double>((const double *)pressure, pressure_level_stride, pressure_is_1d, (const double *)temperature, (const double *)dewpoint, level_stride, n_levels, n_columns, metpy_compat, tb, (double *)out->dcape, (double *)out->start_pressure, (double *)out->start_temperature, (double *)out->parcel_temperature, out->parcel_level_stride, st));
+    ctx->launches += 1;
+    return check_cuda(ctx, cudaGetLastError(), "downdraft_cape kernel launch");
+}
+
 xp_status xp_significant_hail_parameter(xp_context *ctx, const void *mucape, const void *mixing_ratio,
                                         const void *lapse, const void *temp_500, const void *shear,
                                         const void *flh, int64_t n, int32_t dtype, void *ship, void *stream) {

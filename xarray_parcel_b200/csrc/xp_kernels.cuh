@@ -223,6 +223,13 @@ void launch_ship(const T *const *in6, int64_t n, T *out, cudaStream_t stream);
 template <typename T>
 void launch_storm_proxies(const T *const *in13, uint8_t *const *flags9, T *ship, int64_t n, cudaStream_t stream);
 
+// Downdraft CAPE (xp_downdraft.cu, contract in xp_downdraft.cuh): dcape / start pressure / start temperature [N]
+// and the parcel temperature [L][N] with level stride pts; any output may be null.
+template <typename T>
+void launch_downdraft_cape(const T *p, int64_t pls, int p1d, const T *t, const T *td, int64_t ls, int L, int64_t n,
+                           int compat, const Tables &tb, T *dcape, T *p_start, T *t_start, T *parcel_t, int64_t pts,
+                           cudaStream_t stream);
+
 // Table builder (xp_tables.cu): fills index_grid (uint16 [kNP][kNT]) and curves (float
 // [kNAdiabats][kNP] ascending pressure).  `scratch_u32` must hold kNP*kNT uint32.
 void launch_build_tables(uint16_t *index_grid, float *curves, uint32_t *scratch_u32,

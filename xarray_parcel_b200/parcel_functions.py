@@ -36,7 +36,7 @@ __all__ = ["load_moist_adiabat_lookups", "lookup_tables_loaded", "moist_adiabat_
            "parcel_suite", "parcel_suite_chunks", "Dataset", "linear_interp", "log_interp", "lifted_index",
            "deep_convective_index", "isobar_temperature", "lapse_rate", "freezing_level_height",
            "melting_level_height", "wet_bulb_temperature_fast", "wind_shear",
-           "dewpoint_from_specific_humidity", "conv_properties", "min_conv_properties"]
+           "dewpoint_from_specific_humidity", "conv_properties", "min_conv_properties", "downdraft_cape"]
 
 KAPPA = 0.28571428571428564       # metpy.constants.kappa (PF:313)
 
@@ -58,6 +58,10 @@ _ATTRS = {
     "environment_temperature": {"long_name": "Environment temperature", "units": "K"},
     "environment_dewpoint": {"long_name": "Environment dewpoint", "units": "K"},
     "environment_virtual_temperature": {"long_name": "Virtual temperature", "units": "K"},
+    "dcape": {"long_name": "Downdraft convective available potential energy", "units": "J kg$^{-1}$"},
+    "downdraft_start_pressure": {"long_name": "Downdraft source pressure", "units": "hPa"},
+    "downdraft_start_temperature": {"long_name": "Downdraft source wet-bulb temperature", "units": "K"},
+    "downdraft_parcel_temperature": {"long_name": "Downdraft parcel temperature", "units": "K"},
 }
 
 
@@ -1025,6 +1029,30 @@ def wet_bulb_temperature(pressure, temperature, dewpoint, vert_dim="model_level_
                       device=device)
 
 
+def downdraft_cape(pressure, temperature, dewpoint, vert_dim="model_level_number", vert_axis=0, metpy_compat="1.4.1",
+                   profile=False, device=None):
+    """Downdraft CAPE after MetPy's ``downdraft_cape``, on this library's thermodynamics and lookup-table moist
+    adiabat (``xp_downdraft_cape``, one CUDA thread per column; contract in DESIGN.md section 3.12).
+
+    The downdraft starts at the minimum equivalent potential temperature in the 700-500 hPa layer, at its wet-bulb
+    temperature, and descends moist-adiabatically to the surface; ``dcape`` is -Rd times the integral of the
+    environment minus parcel virtual temperature over ln p, not clipped (negative where the parcel is warmer).
+    Columns that do not span 700-500 hPa give NaN.  Returns a Dataset of dcape [J/kg], downdraft_start_pressure
+    [hPa] and downdraft_start_temperature [K] and, with ``profile=True``, downdraft_parcel_temperature on the input
+    levels (NaN above the start and on levels with a NaN input)."""
+    lookup_tables_loaded(device)
+    ctx = _lib.get_context(device)
+    lay, dtype, on_gpu = _layout_of(temperature, vert_dim, vert_axis)
+    t, td, p = _blocks(lay, [temperature, dewpoint, pressure], dtype)
+    r = ctx.downdraft_cape(p, t, td, metpy_compat=metpy_compat, profile=profile)
+    fix = (lambda x: x) if on_gpu else (lambda x: x.cpu())
+    out = {k: lay.wrap_scalar(fix(r[k]), k) for k in _lib.DOWNDRAFT_FIELDS}
+    if profile:
+        out["downdraft_parcel_temperature"] = lay.wrap_profile(fix(r["downdraft_parcel_temperature"]),
+                                                               "downdraft_parcel_temperature", lay.L)
+    return lay.dataset(out)
+
+
 def melting_level_height(pressure, temperature, dewpoint, height, fast=True, vert_dim="model_level_number",
                          vert_axis=0, device=None):
     """PF:2162-2191: lowest height at which the wet-bulb temperature (1/3 rule with fast=True, Normand's
@@ -1124,7 +1152,7 @@ def storm_proxies(dat, device=None):
     return ds
 
 
-def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat):
+def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat, downdraft=False):
     p, t = dat["pressure"], dat["temperature"]
     td = dewpoint_from_specific_humidity(p, t, dat["specific_humidity"], metpy_compat, device=device)
     try:
@@ -1166,6 +1194,8 @@ def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat):
     out["melting_level"], _ = melting_level_height(p, t, td, dat["height_asl"], **kw)
     merge(wind_shear(dat["surface_wind_u"], dat["surface_wind_v"], dat["wind_u"], dat["wind_v"],
                      dat["wind_height_above_surface"], shear_height=6000, **kw))
+    if downdraft:
+        out["dcape"] = downdraft_cape(p, t, td, metpy_compat=metpy_compat, **kw)["dcape"]
     if not min_set and not ignore_nans:                              # PF:1976-1983, 2098-2099
         lay = _Layout(t, vert_dim, vert_axis)
         va = lay.vert_axis if lay.vert_axis is not None else 0
@@ -1193,12 +1223,13 @@ def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat):
 
 
 def conv_properties(dat, vert_dim="model_level_number", ignore_nans=False, vert_axis=0, device=None,
-                    metpy_compat="1.4.1"):
+                    metpy_compat="1.4.1", downdraft=False):
     """PF:1951-2100: MU (250 hPa) and mixed (100, 50 hPa) CAPE/CIN, lifted and deep-convective indices,
     MU mixing ratio, 700-500 hPa lapse rate, 500 hPa temperature, freezing/melting level, 0-6 km shear.
     ``dat``: Dataset/dict with pressure, temperature, specific_humidity, height_asl, wind_u, wind_v,
-    wind_height_above_surface (all [level, ...]) and surface_wind_u, surface_wind_v."""
-    return _conv(dat, vert_dim, vert_axis, device, False, ignore_nans, metpy_compat)
+    wind_height_above_surface (all [level, ...]) and surface_wind_u, surface_wind_v.  ``downdraft=True`` adds
+    ``dcape`` (``downdraft_cape`` on the dewpoint derived from the specific humidity), masked like the rest."""
+    return _conv(dat, vert_dim, vert_axis, device, False, ignore_nans, metpy_compat, downdraft)
 
 
 def min_conv_properties(dat, vert_dim="model_level_number", vert_axis=0, device=None, metpy_compat="1.4.1"):
