@@ -354,6 +354,27 @@ xp_status xp_downdraft_cape(xp_context *ctx, const void *pressure, int64_t press
                             int32_t pressure_is_1d, const void *temperature, const void *dewpoint,
                             int64_t level_stride, int32_t n_levels, int64_t n_columns, int32_t dtype,
                             int32_t metpy_compat, const xp_downdraft_out *out, void *stream);
+/* xp_effective_inflow_layer: the effective inflow layer (Thompson et al. 2007; SHARPpy's effective_inflow_layer) per
+ * column, device memory only.  Contract (DESIGN.md section 3.13): a level is valid when p, T and Td are non-NaN; the
+ * lift from valid level k is the parcel (p_k, T_k, Td_k) on the levels with p <= p_k -- the most-unstable lift with
+ * its level forced to k -- with CAPE / CIN per `opts` (virtual_temperature_correction, lcl_interp_log,
+ * pos_cape_neg_cin, post_zero_cin, metpy_compat; float64 arithmetic; exact_only and mixed_layer_depth have no effect);
+ * a level passes when cape >= min_cape && cin > min_cin (NaN fails).  Gate: the column's most-unstable parcel (over
+ * opts->most_unstable_depth) must pass, else base and top are NaN.  Base: the first valid level from the surface up
+ * that passes (none: NaN).  Top: the valid level just below the first valid level above the base that fails (NaN if
+ * none fails; a one-level layer has top == base).  Outputs, in the input dtype, any may be NULL: base_pressure and
+ * top_pressure [n_columns] in hPa (input pressures, copied exactly); level_cape / level_cin [n_levels][n_columns] with
+ * level stride level_out_stride: the CAPE / CIN of the parcel of every valid level, NaN on invalid levels -- asking
+ * for either lifts EVERY valid level of EVERY column, whatever the gate; base and top are the same in both modes.
+ * The most-unstable selection and the lifts report XP_FLAG_PRESSURES_NOT_UNIQUE and XP_FLAG_TOP_TEMPERATURE_NAN through
+ * xp_take_flags.  XP_ERR_INVALID_ARGUMENT for mem = XP_MEM_HOST, dewpoint_is_specific_humidity = 1, n_levels < 1 or a
+ * non-zero reserved_; XP_ERR_TABLES_NOT_LOADED without the tables. */
+typedef struct xp_effective_out {
+    void *base_pressure, *top_pressure, *level_cape, *level_cin;
+    int64_t level_out_stride;
+} xp_effective_out;
+xp_status xp_effective_inflow_layer(xp_context *ctx, const xp_columns *cols, const xp_options *opts, double min_cape,
+                                    double min_cin, const xp_effective_out *out, void *stream);
 /* significant_hail_parameter (PF:2261-2306): units as the reference's arguments (mixing ratio kg/kg,
  * lapse K/km negative for decreasing temperature, temp_500 K, shear m/s, flh m). */
 xp_status xp_significant_hail_parameter(xp_context *ctx, const void *mucape, const void *mixing_ratio,

@@ -8,8 +8,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(HERE, "libxparcel.so")
 CHECK_LIB_PATH = os.path.join(HERE, "libxparcel_check.so")      # -DXP_BOUNDS_CHECK variant (tests only)
-SOURCES = ["xp_api.cu", "xp_kernels.cu", "xp_list.cu", "xp_tables.cu", "xp_fast.cu", "xp_derived.cu", "xp_layers.cu", "xp_levels.cu", "xp_downdraft.cu"]
-HEADERS = ["xp_math.cuh", "xp_column.cuh", "xp_parcels.cuh", "xp_kernels.cuh", "xp_fast.cuh", "xp_fast_pcol.cuh", "xp_fast6.cuh", "xp_fast7.cuh", "xp_fast_pcol6.cuh", "xp_fast_pcol7.cuh", "xp_kernels_common.cuh", "xp_layers.cuh", "xp_levels.cuh", "xp_downdraft.cuh",
+SOURCES = ["xp_api.cu", "xp_kernels.cu", "xp_list.cu", "xp_tables.cu", "xp_fast.cu", "xp_derived.cu", "xp_layers.cu", "xp_levels.cu", "xp_downdraft.cu", "xp_effective.cu"]
+HEADERS = ["xp_math.cuh", "xp_column.cuh", "xp_parcels.cuh", "xp_kernels.cuh", "xp_fast.cuh", "xp_fast_pcol.cuh", "xp_fast6.cuh", "xp_fast7.cuh", "xp_fast_pcol6.cuh", "xp_fast_pcol7.cuh", "xp_kernels_common.cuh", "xp_layers.cuh", "xp_levels.cuh", "xp_downdraft.cuh", "xp_effective.cuh",
            os.path.join("..", "..", "include", "xparcel.h")]
 NVCC_COMMON = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
                "-Xcompiler", "-fPIC"]
@@ -18,7 +18,8 @@ NVCC_COMMON = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a"
 # float32 fast path (xp_fast.cu) takes no decision inside its error margin, so it may contract.
 PER_FILE_FLAGS = {"xp_fast.cu": [], "xp_api.cu": ["-fmad=false"], "xp_kernels.cu": ["-fmad=false"], "xp_list.cu": ["-fmad=false"],
                   "xp_tables.cu": ["-fmad=false"], "xp_derived.cu": ["-fmad=false"], "xp_layers.cu": ["-fmad=false"],
-                  "xp_levels.cu": ["-fmad=false"], "xp_downdraft.cu": ["-fmad=false"]}
+                  "xp_levels.cu": ["-fmad=false"], "xp_downdraft.cu": ["-fmad=false"],
+                  "xp_effective.cu": ["-fmad=false"]}
 LINK_FLAGS = ["-shared", "-cudart", "static", "-gencode", "arch=compute_100a,code=sm_100a"]
 
 

@@ -66,7 +66,8 @@ EXPORTS = ["xp_version", "xp_create", "xp_destroy", "xp_last_error", "xp_take_fl
            "xp_dry_lapse", "xp_mixing_ratio", "xp_virtual_temperature", "xp_wet_bulb_temperature",
            "xp_significant_hail_parameter", "xp_storm_proxies", "xp_mixed_layer", "xp_mixed_parcel",
            "xp_layer_bounds", "xp_insert_level", "xp_shift_out_nans", "xp_trapz", "xp_valid_data",
-           "xp_find_intersections", "xp_interp1d", "xp_trap_around_zeros", "xp_downdraft_cape"]
+           "xp_find_intersections", "xp_interp1d", "xp_trap_around_zeros", "xp_downdraft_cape",
+           "xp_effective_inflow_layer"]
 
 PROXY_INPUTS = ["mixed_100_cape", "mixed_50_cape", "mu_cape", "shear_magnitude", "mixed_100_lifted_index",
                 "mixed_100_dci", "positive_shear", "mixed_50_cin", "mixed_100_cin", "lapse_rate_700_500",
@@ -103,6 +104,15 @@ DOWNDRAFT_FIELDS = ["dcape", "downdraft_start_pressure", "downdraft_start_temper
 class XpDowndraftOut(ctypes.Structure):
     _fields_ = [("dcape", c_void_p), ("start_pressure", c_void_p), ("start_temperature", c_void_p),
                 ("parcel_temperature", c_void_p), ("parcel_level_stride", c_int64)]
+
+
+EFFECTIVE_FIELDS = ["effective_inflow_base", "effective_inflow_top"]
+EFFECTIVE_LEVEL_FIELDS = ["level_parcel_cape", "level_parcel_cin"]
+
+
+class XpEffectiveOut(ctypes.Structure):
+    _fields_ = [("base_pressure", c_void_p), ("top_pressure", c_void_p), ("level_cape", c_void_p),
+                ("level_cin", c_void_p), ("level_out_stride", c_int64)]
 
 
 class XpProxyInputs(ctypes.Structure):
@@ -208,6 +218,8 @@ def load_library():
                                              c_int64, c_int32, c_int32, ctypes.POINTER(XpZeroAreasOut), c_void_p]
         lib.xp_downdraft_cape.argtypes = [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_int64, c_int32,
                                           c_int64, c_int32, c_int32, ctypes.POINTER(XpDowndraftOut), c_void_p]
+        lib.xp_effective_inflow_layer.argtypes = [c_void_p, ctypes.POINTER(XpColumns), ctypes.POINTER(XpOptions),
+                                                  c_double, c_double, ctypes.POINTER(XpEffectiveOut), c_void_p]
         lib.xp_launch_count.argtypes = [c_void_p]
         lib.xp_launch_count.restype = ctypes.c_uint64
         lib.xp_last_kernel_ms.argtypes = [c_void_p, ctypes.POINTER(ctypes.c_float)]
@@ -633,6 +645,28 @@ class Context:
                                         temperature.data_ptr(), dewpoint.data_ptr(), temperature.stride(0), L, N,
                                         _dtype_code(temperature), compat, ctypes.byref(o), self._stream())
         self._check(st, "xp_downdraft_cape")
+        return res
+
+    def effective_inflow_layer(self, p, t, td, options=None, min_cape=100.0, min_cin=-250.0, profile=False,
+                               outputs=None):
+        """Effective inflow layer (xp_effective_inflow_layer) of the device columns ``t`` / ``td`` [L, N] on ``p``
+        ([L, N] or a shared [L]).  Returns a dict of the EFFECTIVE_FIELDS [N] (base and top pressure) and, with
+        ``profile``, the EFFECTIVE_LEVEL_FIELDS [L, N] (CAPE / CIN of the parcel of every level; this lifts every
+        valid level of every column).  ``outputs`` (a subset of those names) leaves the others uncomputed (NULL in the
+        call).  ``options``: make_options(...) (most_unstable_depth selects the gate's parcel)."""
+        opts = options if options is not None else make_options()
+        cols, L, N = self._columns(p, t, td)
+        names = list(EFFECTIVE_FIELDS) + (list(EFFECTIVE_LEVEL_FIELDS) if profile else [])
+        if outputs is not None:
+            names = [n for n in names if n in outputs]
+        res = {n: torch.empty((L, N) if n in EFFECTIVE_LEVEL_FIELDS else (N,), dtype=t.dtype, device=t.device)
+               for n in names}
+        ptr = {n: res[n].data_ptr() if n in res else None for n in EFFECTIVE_FIELDS + EFFECTIVE_LEVEL_FIELDS}
+        o = XpEffectiveOut(ptr["effective_inflow_base"], ptr["effective_inflow_top"], ptr["level_parcel_cape"],
+                           ptr["level_parcel_cin"], N)
+        st = self.lib.xp_effective_inflow_layer(self.handle, ctypes.byref(cols), ctypes.byref(opts), float(min_cape),
+                                                float(min_cin), ctypes.byref(o), self._stream())
+        self._check(st, "xp_effective_inflow_layer")
         return res
     # ---- level primitives (xp_levels.cu) ---------------------------------------------------------------
     @staticmethod

@@ -157,6 +157,27 @@ xp_status validate_cols(xp_context *ctx, const xp_columns *c) {
     return XP_OK;
 }
 
+// The context's scratch buffer of `stream`, grown to at least `need` bytes.  One buffer per stream in use: a call
+// may reuse it as soon as the previous call on the same stream is done with it, which stream order guarantees.
+cudaError_t stream_scratch(xp_context *ctx, cudaStream_t stream, size_t need, void **out) {
+    if (!ctx->scratch.count(stream) && ctx->scratch.size() >= kMaxScratchStreams) {
+        // bound the per-stream scratch map: drop the buffers of the other streams (after their work is done)
+        for (auto &kv : ctx->scratch) {
+            if (kv.second.ptr) { cudaStreamSynchronize(kv.first); cudaFree(kv.second.ptr); }
+        }
+        ctx->scratch.clear();
+    }
+    xp_context::Scratch &sc = ctx->scratch[stream];
+    if (sc.bytes < need) {
+        if (sc.ptr) { cudaStreamSynchronize(stream); cudaFree(sc.ptr); sc.ptr = nullptr; sc.bytes = 0; }
+        const cudaError_t e = cudaMalloc(&sc.ptr, need);
+        if (e != cudaSuccess) return e;
+        sc.bytes = need;
+    }
+    *out = sc.ptr;
+    return cudaSuccess;
+}
+
 // Launch the fused kernel on device-resident columns.
 template <typename T>
 xp_status run_device(xp_context *ctx, const xp_columns *cols, int kind_mask,
@@ -175,22 +196,10 @@ xp_status run_device(xp_context *ctx, const xp_columns *cols, int kind_mask,
     if constexpr (std::is_same<T, float>::value) {
         const ColsArg<float> ca = to_cols<float>(cols, o);
         if (!o.exact_only && cols->n_columns > 0 && fast_eligible(ca, kind_mask, oa, o)) {
-            if (!ctx->scratch.count(stream) && ctx->scratch.size() >= kMaxScratchStreams) {
-                // bound the per-stream scratch map: drop the buffers of the other streams (after their work is done)
-                for (auto &kv : ctx->scratch) {
-                    if (kv.second.ptr) { cudaStreamSynchronize(kv.first); cudaFree(kv.second.ptr); }
-                }
-                ctx->scratch.clear();
-            }
-            xp_context::Scratch &sc = ctx->scratch[stream];
-            const size_t need = fast_scratch_bytes(cols->n_columns);
-            if (sc.bytes < need) {
-                if (sc.ptr) { cudaStreamSynchronize(stream); cudaFree(sc.ptr); sc.ptr = nullptr; sc.bytes = 0; }
-                XP_CUDA(ctx, cudaMalloc(&sc.ptr, need));
-                sc.bytes = need;
-            }
+            void *sp = nullptr;
+            XP_CUDA(ctx, stream_scratch(ctx, stream, fast_scratch_bytes(cols->n_columns), &sp));
             if (time_it) { cudaEventRecord(ctx->ev0, stream); g_event_before_list = ctx->ev_mid; }
-            const int nl = launch_suite_fast(ca, tb, o, kind_mask, oa, sc.ptr, ctx->d_flags, ctx->sm_count, stream);
+            const int nl = launch_suite_fast(ca, tb, o, kind_mask, oa, sp, ctx->d_flags, ctx->sm_count, stream);
             g_event_before_list = nullptr;
             if (nl < 0) return check_cuda(ctx, cudaGetLastError(), "fast suite shared-memory attribute");
             ctx->launches += nl;
@@ -203,21 +212,10 @@ xp_status run_device(xp_context *ctx, const xp_columns *cols, int kind_mask,
     if constexpr (std::is_same<T, double>::value) {
         // float64 columns on a shared pressure axis, default options: the same fast kernel (launch_suite_fast_f64)
         if (!o.exact_only && cols->n_columns > 0 && cols->pressure_is_1d && !(kind_mask & kEX)) {
-            if (!ctx->scratch.count(stream) && ctx->scratch.size() >= kMaxScratchStreams) {
-                for (auto &kv : ctx->scratch) {
-                    if (kv.second.ptr) { cudaStreamSynchronize(kv.first); cudaFree(kv.second.ptr); }
-                }
-                ctx->scratch.clear();
-            }
-            xp_context::Scratch &sc = ctx->scratch[stream];
-            const size_t need = fast_scratch_bytes(cols->n_columns);
-            if (sc.bytes < need) {
-                if (sc.ptr) { cudaStreamSynchronize(stream); cudaFree(sc.ptr); sc.ptr = nullptr; sc.bytes = 0; }
-                XP_CUDA(ctx, cudaMalloc(&sc.ptr, need));
-                sc.bytes = need;
-            }
+            void *sp = nullptr;
+            XP_CUDA(ctx, stream_scratch(ctx, stream, fast_scratch_bytes(cols->n_columns), &sp));
             if (time_it) { cudaEventRecord(ctx->ev0, stream); g_event_before_list = ctx->ev_mid; }
-            const int nl = launch_suite_fast_f64(to_cols<double>(cols, o), tb, o, kind_mask, oa, sc.ptr, ctx->d_flags,
+            const int nl = launch_suite_fast_f64(to_cols<double>(cols, o), tb, o, kind_mask, oa, sp, ctx->d_flags,
                                                  ctx->sm_count, stream);
             g_event_before_list = nullptr;
             if (nl == -1) return check_cuda(ctx, cudaGetLastError(), "fast suite shared-memory attribute");
@@ -1129,6 +1127,47 @@ xp_status xp_downdraft_cape(xp_context *ctx, const void *pressure, int64_t press
                 launch_downdraft_cape<double>((const double *)pressure, pressure_level_stride, pressure_is_1d, (const double *)temperature, (const double *)dewpoint, level_stride, n_levels, n_columns, metpy_compat, tb, (double *)out->dcape, (double *)out->start_pressure, (double *)out->start_temperature, (double *)out->parcel_temperature, out->parcel_level_stride, st));
     ctx->launches += 1;
     return check_cuda(ctx, cudaGetLastError(), "downdraft_cape kernel launch");
+}
+
+// Effective inflow layer, contract in include/xparcel.h and xp_effective.cuh (DESIGN.md section 3.13).
+xp_status xp_effective_inflow_layer(xp_context *ctx, const xp_columns *cols, const xp_options *opts, double min_cape,
+                                    double min_cin, const xp_effective_out *out, void *stream) {
+    if (!ctx) return XP_ERR_INVALID_ARGUMENT;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    xp_status st = validate_cols(ctx, cols);
+    if (st != XP_OK) return st;
+    if (!out) return fail(ctx, XP_ERR_INVALID_ARGUMENT, "out is NULL");
+    if (cols->mem != XP_MEM_DEVICE)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "effective_inflow_layer: device memory only (mem = XP_MEM_DEVICE)");
+    if (cols->dewpoint_is_specific_humidity)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "effective_inflow_layer: dewpoint_is_specific_humidity is not supported");
+    if (cols->reserved_ != 0) return fail(ctx, XP_ERR_INVALID_ARGUMENT, "reserved_ must be 0");
+    if (!ctx->tables) return fail(ctx, XP_ERR_TABLES_NOT_LOADED, "Call load_moist_adiabat_lookups first.");
+    if (cols->n_columns == 0) return XP_OK;
+    if ((out->level_cape || out->level_cin) && out->level_out_stride < cols->n_columns)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "effective_inflow_layer: level_out_stride must be >= n_columns");
+    if (cols->n_columns > (int64_t)1 << 40)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "effective_inflow_layer: more than 2^40 columns");
+    if (!out->base_pressure && !out->top_pressure && !out->level_cape && !out->level_cin) return XP_OK;
+    DeviceGuard guard(ctx->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    const Opts o = to_opts(ctx, opts);
+    void *scratch = nullptr;
+    XP_CUDA(ctx, stream_scratch(ctx, s, effective_scratch_bytes(cols->n_columns), &scratch));
+    if (ctx->last_fast_stream == s) ctx->last_was_fast = false;     // its fix-up list count is gone with the scratch
+    const Tables tb = {ctx->d_index, ctx->d_curves};
+    int rc;
+    if (cols->dtype == XP_F32)
+        rc = launch_effective<float>(to_cols<float>(cols, o), tb, o, min_cape, min_cin, (float *)out->base_pressure,
+                                     (float *)out->top_pressure, (float *)out->level_cape, (float *)out->level_cin,
+                                     out->level_out_stride, ctx->d_flags, scratch, ctx->sm_count, s);
+    else
+        rc = launch_effective<double>(to_cols<double>(cols, o), tb, o, min_cape, min_cin, (double *)out->base_pressure,
+                                      (double *)out->top_pressure, (double *)out->level_cape, (double *)out->level_cin,
+                                      out->level_out_stride, ctx->d_flags, scratch, ctx->sm_count, s);
+    if (rc < 0) return fail(ctx, XP_ERR_INVALID_ARGUMENT, "effective_inflow_layer: too many levels on a shared axis");
+    ctx->launches += 2;
+    return check_cuda(ctx, cudaGetLastError(), "effective_inflow_layer kernel launch");
 }
 
 xp_status xp_significant_hail_parameter(xp_context *ctx, const void *mucape, const void *mixing_ratio,

@@ -230,6 +230,16 @@ void launch_downdraft_cape(const T *p, int64_t pls, int p1d, const T *t, const T
                            int compat, const Tables &tb, T *dcape, T *p_start, T *t_start, T *parcel_t, int64_t pts,
                            cudaStream_t stream);
 
+// Effective inflow layer (xp_effective.cu, contract in xp_effective.cuh): base / top pressure [N] and, when either
+// level output is non-null (all-levels mode), the CAPE / CIN of the parcel of every level [L][N] with level stride
+// lls; any output may be null.  `scratch` must hold effective_scratch_bytes(n) bytes and must not be shared by launches
+// in flight.  Returns 0, or -1 when a shared pressure axis has too many levels for its ln p table.
+size_t effective_scratch_bytes(int64_t n);
+template <typename T>
+int launch_effective(const ColsArg<T> &cols, const Tables &tb, const Opts &o, double min_cape, double min_cin,
+                     T *base, T *top, T *lcape, T *lcin, int64_t lls, uint32_t *flags, void *scratch, int sm_count,
+                     cudaStream_t stream);
+
 // Table builder (xp_tables.cu): fills index_grid (uint16 [kNP][kNT]) and curves (float
 // [kNAdiabats][kNP] ascending pressure).  `scratch_u32` must hold kNP*kNT uint32.
 void launch_build_tables(uint16_t *index_grid, float *curves, uint32_t *scratch_u32,

@@ -36,7 +36,8 @@ __all__ = ["load_moist_adiabat_lookups", "lookup_tables_loaded", "moist_adiabat_
            "parcel_suite", "parcel_suite_chunks", "Dataset", "linear_interp", "log_interp", "lifted_index",
            "deep_convective_index", "isobar_temperature", "lapse_rate", "freezing_level_height",
            "melting_level_height", "wet_bulb_temperature_fast", "wind_shear",
-           "dewpoint_from_specific_humidity", "conv_properties", "min_conv_properties", "downdraft_cape"]
+           "dewpoint_from_specific_humidity", "conv_properties", "min_conv_properties", "downdraft_cape",
+           "effective_inflow_layer"]
 
 KAPPA = 0.28571428571428564       # metpy.constants.kappa (PF:313)
 
@@ -62,6 +63,10 @@ _ATTRS = {
     "downdraft_start_pressure": {"long_name": "Downdraft source pressure", "units": "hPa"},
     "downdraft_start_temperature": {"long_name": "Downdraft source wet-bulb temperature", "units": "K"},
     "downdraft_parcel_temperature": {"long_name": "Downdraft parcel temperature", "units": "K"},
+    "effective_inflow_base": {"long_name": "Effective inflow layer base pressure", "units": "hPa"},
+    "effective_inflow_top": {"long_name": "Effective inflow layer top pressure", "units": "hPa"},
+    "level_parcel_cape": {"long_name": "CAPE of the parcel lifted from each level", "units": "J kg$^{-1}$"},
+    "level_parcel_cin": {"long_name": "CIN of the parcel lifted from each level", "units": "J kg$^{-1}$"},
 }
 
 
@@ -1053,6 +1058,37 @@ def downdraft_cape(pressure, temperature, dewpoint, vert_dim="model_level_number
     return lay.dataset(out)
 
 
+def effective_inflow_layer(pressure, temperature, dewpoint, vert_dim="model_level_number", vert_axis=0, min_cape=100,
+                           min_cin=-250, most_unstable_depth=300, profile=False, device=None, **kwargs):
+    """The effective inflow layer (Thompson et al. 2007, SHARPpy's ``effective_inflow_layer``) on this library's
+    parcel lift (``xp_effective_inflow_layer``; contract in DESIGN.md section 3.13).
+
+    A level is valid when pressure, temperature and dewpoint are all non-NaN.  The parcel of a valid level is lifted
+    over the levels above it, with CAPE / CIN as ``cape_cin`` computes them (``kwargs``: its options,
+    ``virtual_temperature_correction``, ``lcl_interp``, ``pos_cape_neg_cin``, ``post_zero_cin``, ``metpy_compat``),
+    and passes when CAPE >= ``min_cape`` and CIN > ``min_cin`` [J/kg].  If the most-unstable parcel (over
+    ``most_unstable_depth`` hPa) fails, the column has no layer.  Otherwise the base is the first passing level from
+    the surface up and the top is the last passing level before the first failing one above it.  Returns a Dataset
+    of effective_inflow_base and effective_inflow_top [hPa] (NaN: no layer) and, with ``profile=True``,
+    level_parcel_cape and level_parcel_cin on the input levels (NaN on invalid levels), which lifts every valid
+    level of every column."""
+    lookup_tables_loaded(device)
+    ctx = _lib.get_context(device)
+    lay, dtype, on_gpu = _layout_of(temperature, vert_dim, vert_axis)
+    dev = f"cuda:{ctx.device}"
+    t, td, p = [b.to(dev).contiguous() for b in _blocks(lay, [temperature, dewpoint, pressure], dtype)]
+    opts = _lib.make_options(most_unstable_depth=most_unstable_depth, **_options(kwargs))
+    _clear_flags(ctx)
+    r = ctx.effective_inflow_layer(p, t, td, options=opts, min_cape=min_cape, min_cin=min_cin, profile=profile)
+    _check_flags(ctx)
+    fix = (lambda x: x) if on_gpu else (lambda x: x.cpu())
+    out = {k: lay.wrap_scalar(fix(r[k]), k) for k in _lib.EFFECTIVE_FIELDS}
+    if profile:
+        for k in _lib.EFFECTIVE_LEVEL_FIELDS:
+            out[k] = lay.wrap_profile(fix(r[k]), k, lay.L)
+    return lay.dataset(out)
+
+
 def melting_level_height(pressure, temperature, dewpoint, height, fast=True, vert_dim="model_level_number",
                          vert_axis=0, device=None):
     """PF:2162-2191: lowest height at which the wet-bulb temperature (1/3 rule with fast=True, Normand's
@@ -1152,7 +1188,7 @@ def storm_proxies(dat, device=None):
     return ds
 
 
-def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat, downdraft=False):
+def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat, downdraft=False, effective=False):
     p, t = dat["pressure"], dat["temperature"]
     td = dewpoint_from_specific_humidity(p, t, dat["specific_humidity"], metpy_compat, device=device)
     try:
@@ -1196,6 +1232,10 @@ def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat, 
                      dat["wind_height_above_surface"], shear_height=6000, **kw))
     if downdraft:
         out["dcape"] = downdraft_cape(p, t, td, metpy_compat=metpy_compat, **kw)["dcape"]
+    if effective:
+        eff = effective_inflow_layer(p, t, td, metpy_compat=metpy_compat, **kw)
+        for k in _lib.EFFECTIVE_FIELDS:
+            out[k] = eff[k]
     if not min_set and not ignore_nans:                              # PF:1976-1983, 2098-2099
         lay = _Layout(t, vert_dim, vert_axis)
         va = lay.vert_axis if lay.vert_axis is not None else 0
@@ -1223,13 +1263,15 @@ def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat, 
 
 
 def conv_properties(dat, vert_dim="model_level_number", ignore_nans=False, vert_axis=0, device=None,
-                    metpy_compat="1.4.1", downdraft=False):
+                    metpy_compat="1.4.1", downdraft=False, effective=False):
     """PF:1951-2100: MU (250 hPa) and mixed (100, 50 hPa) CAPE/CIN, lifted and deep-convective indices,
     MU mixing ratio, 700-500 hPa lapse rate, 500 hPa temperature, freezing/melting level, 0-6 km shear.
     ``dat``: Dataset/dict with pressure, temperature, specific_humidity, height_asl, wind_u, wind_v,
     wind_height_above_surface (all [level, ...]) and surface_wind_u, surface_wind_v.  ``downdraft=True`` adds
-    ``dcape`` (``downdraft_cape`` on the dewpoint derived from the specific humidity), masked like the rest."""
-    return _conv(dat, vert_dim, vert_axis, device, False, ignore_nans, metpy_compat, downdraft)
+    ``dcape`` (``downdraft_cape`` on the dewpoint derived from the specific humidity), masked like the rest;
+    ``effective=True`` adds ``effective_inflow_base`` and ``effective_inflow_top`` (``effective_inflow_layer`` with
+    its defaults on that dewpoint), masked the same way."""
+    return _conv(dat, vert_dim, vert_axis, device, False, ignore_nans, metpy_compat, downdraft, effective)
 
 
 def min_conv_properties(dat, vert_dim="model_level_number", vert_axis=0, device=None, metpy_compat="1.4.1"):
