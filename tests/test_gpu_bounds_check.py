@@ -4,7 +4,9 @@
 the fast kernels -- shared-memory stash and coefficient table, the uncertain-column list, the 32-bit T/Td offsets --
 and traps on a violation, which surfaces as a CUDA error in the child process below.  The child drives the fast
 kernels over the awkward inputs: NaN-laden and all-NaN columns, saturated parcels, 3-level and 56-level axes, axes
-reaching above the table top, column counts that are not a multiple of the tile, specific-humidity input."""
+reaching above the table top, column counts that are not a multiple of the tile, specific-humidity input; and the
+regime columns of tests/regime_columns.py -- cold parcels, surfaces above 1100 hPa and model tops at 0.01 hPa (table rows
+outside the segments, every column on the fix-up list: three lists of N items), ERA5 levels masked below ground."""
 
 import os
 import subprocess
@@ -16,9 +18,11 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CHECK_LIB = os.path.join(ROOT, "xarray_parcel_b200", "libxparcel_check.so")
 
 CHILD = r"""
-import sys
+import os, sys
 sys.path.insert(0, %r)
+sys.path.insert(0, os.path.join(sys.path[0], "tests"))
 import numpy as np, torch
+import regime_columns as rc
 from xarray_parcel_b200 import _lib, synth
 ctx = _lib.get_context(0)
 ctx.tables_build()
@@ -45,6 +49,13 @@ run(p, t, (w / (1 + w)).contiguous(), specific_humidity=True); n_cases += 1
 # profile rows from the per-column-pressure kernel
 p, t, td = synth.model_level_columns(20000, 90, seed=9)
 r = ctx.cape_cin(p.cuda(), t.cuda(), td.cuda(), kinds=("mu",), profile=True); torch.cuda.synchronize(); n_cases += 1
+# regime columns: the table route (three kinds), the gather route (one kind), the shared axis
+for regime, kw in (("cold", {}), ("above_1100", {}), ("synth_like", dict(levels=137, p_top=0.01)),
+                   ("synth_like", dict(levels=150, p_top=0.01)), ("masked", dict(layout="era5_masked"))):
+    p, t, td, _ = rc.columns(regime, 3001, seed=7, **kw)
+    p, t, td = (torch.from_numpy(x) for x in (p, t, td))
+    run(p, t, td); n_cases += 1
+    r = ctx.cape_cin(p.cuda(), t.cuda(), td.cuda(), kinds=("mu",)); torch.cuda.synchronize(); n_cases += 1
 print("BOUNDS_CHECK_OK", n_cases)
 """
 
