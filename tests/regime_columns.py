@@ -5,11 +5,12 @@ model top at 20 hPa.  Users' grids go further: high terrain (the Tibetan plateau
 hPa and 220-250 K), moist heat with surface dewpoints near 308 K, model tops at 0.01 hPa (IFS L137, ERA5 model levels),
 sea-level extrapolations above 1100 hPa and ERA5 pressure-level data with the below-ground levels masked to NaN.  Those
 inputs take other routes through the fast kernels -- the table rows outside segment A, every column handed over to the
-float64 fix-up -- so the GPU tests draw them from here.
+float64 fix-up -- and through the downdraft and effective-layer kernels, so the GPU tests draw them from here.
 
 Every regime gives float32 level-major ``[L, N]`` temperature and dewpoint.  ``layout="model"`` puts them on per-column
 hybrid-sigma pressure ``[L, N]``; ``"era5"`` on the 37 shared ERA5 levels with the below-ground levels extrapolated
-(6.5 K/km, constant dewpoint depression) as ERA5 does; ``"era5_masked"`` the same with the below-ground levels NaN.
+(6.5 K/km, constant dewpoint depression) as ERA5 does; ``"era5_masked"`` the same with the below-ground levels NaN;
+``"axis"`` on a deep shared axis of ``levels`` levels up to ``p_top``, extrapolated below ground.
 """
 
 import numpy as np
@@ -75,9 +76,18 @@ def _model_pressure(p0, levels, p_top):
     return np.exp(np.log(p0)[None, :] * sigma[:, None] + np.log(p_top) * (1.0 - sigma[:, None]))
 
 
+def axis_pressure(regime, levels, p_top):
+    """The shared axis of ``layout="axis"``: ``levels`` pressures [hPa] spaced as the hybrid-sigma levels of a column
+    whose surface is the regime's highest surface pressure (1150 hPa where columns lie above 1100 hPa)."""
+    spec = REGIMES[regime]
+    p_bottom = 1150.0 if spec.get("above_1100") else spec["p0"][1]
+    return _model_pressure(np.array([p_bottom]), levels, p_top)[:, 0]
+
+
 def columns(regime, n, seed, layout="model", levels=70, p_top=20.0):
-    """(p, T, Td, p0) of ``n`` columns of ``regime``: float32 arrays (p [L, N] for ``layout="model"``, [37] otherwise)
-    and the float64 surface pressure [N] the columns were drawn for."""
+    """(p, T, Td, p0) of ``n`` columns of ``regime``: float32 arrays (p [L, N] for ``layout="model"``, [37] for the
+    ERA5 layouts, [levels] for ``layout="axis"``) and the float64 surface pressure [N] the columns were drawn for.
+    ``"axis"`` is a deep shared axis (``axis_pressure``) with the below-ground levels extrapolated as in ``"era5"``."""
     spec = REGIMES[regime]
     rng = np.random.default_rng(seed)
     p0 = _surface_pressure(spec, n, rng)
@@ -85,7 +95,12 @@ def columns(regime, n, seed, layout="model", levels=70, p_top=20.0):
         p32 = _model_pressure(p0, levels, p_top).astype(np.float32)
         assert (np.diff(p32, axis=0) < 0).all(), "pressure must decrease strictly with level"
         t, td = _thermo(p32.astype(np.float64), p0, spec, rng)
+    elif layout == "axis":
+        p32 = axis_pressure(regime, levels, p_top).astype(np.float32)
+        assert (np.diff(p32) < 0).all(), "pressure must decrease strictly with level"
+        t, td = _thermo(np.broadcast_to(p32.astype(np.float64)[:, None], (levels, n)), p0, spec, rng)
     else:
+        assert layout in ("era5", "era5_masked"), layout
         p32 = ERA5_LEVELS_HPA.astype(np.float32)
         t, td = _thermo(np.broadcast_to(ERA5_LEVELS_HPA[:, None], (37, n)), p0, spec, rng)
     t32 = t.astype(np.float32)

@@ -6,7 +6,10 @@ and traps on a violation, which surfaces as a CUDA error in the child process be
 kernels over the awkward inputs: NaN-laden and all-NaN columns, saturated parcels, 3-level and 56-level axes, axes
 reaching above the table top, column counts that are not a multiple of the tile, specific-humidity input; and the
 regime columns of tests/regime_columns.py -- cold parcels, surfaces above 1100 hPa and model tops at 0.01 hPa (table rows
-outside the segments, every column on the fix-up list: three lists of N items), ERA5 levels masked below ground."""
+outside the segments, every column on the fix-up list: three lists of N items), ERA5 levels masked below ground.  DCAPE
+and the effective inflow layer (search and all-levels mode, the gate's column list) run on regime columns too: the
+staged per-column readers (40 and 16 levels), the 0.01 hPa top at 137 levels per column and on a shared axis, surfaces
+above 1100 hPa and masked ERA5 levels."""
 
 import os
 import subprocess
@@ -56,6 +59,17 @@ for regime, kw in (("cold", {}), ("above_1100", {}), ("synth_like", dict(levels=
     p, t, td = (torch.from_numpy(x) for x in (p, t, td))
     run(p, t, td); n_cases += 1
     r = ctx.cape_cin(p.cuda(), t.cuda(), td.cuda(), kinds=("mu",)); torch.cuda.synchronize(); n_cases += 1
+# DCAPE and the effective layer in both modes, float32 and float64
+for regime, kw in (("terrain", dict(levels=40)), ("terrain", dict(levels=16)), ("synth_like", dict(levels=137, p_top=0.01)),
+                   ("synth_like", dict(layout="axis", levels=137, p_top=0.01)), ("above_1100", {}),
+                   ("masked", dict(layout="era5_masked"))):
+    p, t, td, _ = rc.columns(regime, 3001, seed=8, **kw)
+    for dt in (torch.float32, torch.float64):
+        pg, tg, tdg = (torch.from_numpy(x).to(dt).cuda() for x in (p, t, td))
+        ctx.downdraft_cape(pg, tg, tdg, profile=True)
+        ctx.effective_inflow_layer(pg, tg, tdg)
+        ctx.effective_inflow_layer(pg, tg, tdg, profile=True)
+        torch.cuda.synchronize(); n_cases += 1
 print("BOUNDS_CHECK_OK", n_cases)
 """
 

@@ -41,9 +41,11 @@ def _np(x):
     return np.asarray(x.cpu().numpy() if isinstance(x, torch.Tensor) else x, dtype=np.float64)
 
 
-def _compare(got, P, T, D, tables, compat="1.4.1", float32=False):
-    """float64: the oracle at 1e-9; float32: the oracle fed the float32 inputs, rounded to float32, at 2 ulp."""
-    ora = dd.downdraft_cape(P, T, D, op.Options(op.MoistLapseLUT(tables), metpy_compat=compat))
+def _compare(got, P, T, D, tables, compat="1.4.1", float32=False, ora=None):
+    """float64: the oracle at 1e-9; float32: the oracle fed the float32 inputs, rounded to float32, at 2 ulp.  ``ora``:
+    the oracle's float64 result on these inputs and ``compat``, when the caller has it already."""
+    if ora is None:
+        ora = dd.downdraft_cape(P, T, D, op.Options(op.MoistLapseLUT(tables), metpy_compat=compat))
     if float32:
         ora = {k: v.astype(np.float32).astype(np.float64) for k, v in ora.items()}
     g = {k: _np(v) for k, v in got.items()}

@@ -41,11 +41,13 @@ def _np(x):
     return np.asarray(x.cpu().numpy() if isinstance(x, torch.Tensor) else x, dtype=np.float64)
 
 
-def _compare(got, P, T, D, tables, float32=False):
+def _compare(got, P, T, D, tables, float32=False, ora=None):
     """Levels: the oracle at 1e-9 (float64) or 2 ulp of float32 (the oracle fed the same float32 inputs), saturated
     starts excused.  Base / top: the search on the GPU's own level values where they were returned, and the oracle's
-    base / top except in columns with a level value within the comparison tolerance of a threshold."""
-    ora = eo.effective_inflow_layer(P, T, D, op.Options(op.MoistLapseLUT(tables)))
+    base / top except in columns with a level value within the comparison tolerance of a threshold.  ``ora``: the
+    oracle's float64 result on these inputs, when the caller has it already."""
+    if ora is None:
+        ora = eo.effective_inflow_layer(P, T, D, op.Options(op.MoistLapseLUT(tables)))
     g = {k: _np(v) for k, v in got.items()}
     valid = eo.valid_levels(P, T, D)
     rtol = 2.4e-7 if float32 else 1e-9
