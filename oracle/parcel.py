@@ -782,10 +782,11 @@ def wind_shear(surface_wind_u, surface_wind_v, wind_u, wind_v, height, shear_hei
                 "positive_shear": np.sqrt(hi["u"] ** 2 + hi["v"] ** 2) > np.sqrt(surface_wind_u ** 2 + surface_wind_v ** 2)}
 
 
-def conv_properties(dat, opts, min_set=False):
+def conv_properties(dat, opts, min_set=False, ignore_nans=False):
     """PF:1951-2100 (min_set: PF:1872-1949 min_conv_properties).  ``dat``: dict of [L,N] arrays pressure,
     temperature, specific_humidity, height_asl, wind_u, wind_v, wind_height_above_surface and [N] arrays
-    surface_wind_u, surface_wind_v.  Returns a flat dict of [N] arrays."""
+    surface_wind_u, surface_wind_v.  ``ignore_nans`` skips the mask of columns with a NaN input (PF:1976-1983),
+    which min_set never applies.  Returns a flat dict of [N] arrays."""
     p, t = dat["pressure"], dat["temperature"]
     td = th.dewpoint_from_specific_humidity(p, t, dat["specific_humidity"], opts.metpy_compat)
     out = {}
@@ -813,7 +814,7 @@ def conv_properties(dat, opts, min_set=False):
     out["melting_level"] = freezing_level_height(wet_bulb_temperature_fast(t, td), dat["height_asl"])
     out.update(wind_shear(dat["surface_wind_u"], dat["surface_wind_v"], dat["wind_u"], dat["wind_v"],
                           dat["wind_height_above_surface"], 6000))
-    if not min_set:
+    if not min_set and not ignore_nans:
         valid = ~(np.isnan(td).any(0) | np.isnan(p).any(0) | np.isnan(t).any(0) |
                   np.isnan(dat["specific_humidity"]).any(0))                      # PF:1976-1983, 2098-2099
         out = {k: np.where(valid, v, np.nan) for k, v in out.items()}

@@ -112,6 +112,54 @@ def columns(regime, n, seed, layout="model", levels=70, p_top=20.0):
     return p32, np.ascontiguousarray(t32), np.ascontiguousarray(td32), p0
 
 
+def conv_fields(p, t, td, p0, seed, dry_top_every=53, negative_q_every=211):
+    """The ``conv_properties`` input dict of a regime's columns ``(p, T, Td, p0)``, float32 throughout.
+
+    specific_humidity from Td (NaN where Td is masked).  height_asl is hypsometric on the float64 virtual temperature
+    from a surface at 7.5 km * ln(1013.25 / p0) and stays finite on extrapolated and masked levels, as ERA5 geopotential
+    does (a masked level takes the virtual temperature of the lowest valid level).  Winds are seeded sheared profiles,
+    NaN where T is masked; wind_height_above_surface = height_asl - surface height, negative below ground;
+    surface_wind_u / _v are per-column.  Every ``dry_top_every``-th column (from column 3) has q exactly 0 on its top two
+    levels and every ``negative_q_every``-th (from column 7) -1e-7 there, as model output can carry both."""
+    rng = np.random.default_rng(seed)
+    L, n = t.shape
+    q = specific_humidity(p, td)
+    # a warm layer (up to +8 K, 800 m deep, 0.3-3 km above the surface) in every fourth column: inversions that cross
+    # 0 C several times where the column is near freezing there
+    P = np.broadcast_to(np.asarray(p, np.float64).reshape(L, -1), (L, n))
+    z = 7.5 * np.log(p0[None, :] / P)
+    bump = rng.uniform(2.0, 8.0, n) * (np.arange(n) % 4 == 1)
+    t = (t + bump[None, :] * np.clip(1.0 - np.abs(z - rng.uniform(0.3, 3.0, n)[None, :]) / 0.4, 0.0, None)).astype(
+        np.float32)
+    q[-2:, 3::dry_top_every] = 0.0
+    q[-2:, 7::negative_q_every] = -1e-7
+    T = t.astype(np.float64)
+    Q = np.nan_to_num(q.astype(np.float64), nan=0.0)
+    tv = T * (1.0 + 0.608 * Q / (1.0 - Q))
+    valid = ~np.isnan(tv)
+    first = np.argmax(valid, axis=0)                                   # lowest valid level (0 if none)
+    lowest = np.where(valid.any(axis=0), tv[first, np.arange(n)], 250.0)
+    for k in range(L - 1, -1, -1):                                     # masked levels: the lowest valid Tv below
+        tv[k] = np.where(np.isnan(tv[k]), lowest, tv[k])
+    rd_g = 287.04749097718457 / 9.80665
+    z_sfc = 7500.0 * np.log(1013.25 / p0)
+    h = np.empty((L, n))
+    h[0] = z_sfc + rd_g * tv[0] * np.log(p0 / P[0])                   # negative offset when level 0 is below ground
+    for k in range(1, L):
+        h[k] = h[k - 1] + rd_g * 0.5 * (tv[k - 1] + tv[k]) * np.log(P[k - 1] / P[k])
+    agl = h - z_sfc[None, :]
+    km = np.clip(agl, 0.0, None) / 1000.0
+    u = rng.normal(3.0, 5.0, n)[None, :] + rng.uniform(-1.0, 6.0, n)[None, :] * km + rng.normal(0.0, 1.5, (L, n))
+    v = rng.normal(0.0, 5.0, n)[None, :] + rng.uniform(-3.0, 3.0, n)[None, :] * km + rng.normal(0.0, 1.5, (L, n))
+    masked = np.isnan(t)
+    u[masked] = np.nan
+    v[masked] = np.nan
+    f32 = lambda x: np.ascontiguousarray(x, dtype=np.float32)                  # noqa: E731
+    return {"pressure": np.asarray(p, np.float32), "temperature": f32(t), "specific_humidity": f32(q),
+            "height_asl": f32(h), "wind_u": f32(u), "wind_v": f32(v), "wind_height_above_surface": f32(agl),
+            "surface_wind_u": f32(rng.normal(2.0, 4.0, n)), "surface_wind_v": f32(rng.normal(0.0, 4.0, n))}
+
+
 def specific_humidity(p, td):
     """float32 specific humidity [kg/kg] of dewpoint ``td`` [K] at ``p`` [hPa] (Bolton's vapour pressure)."""
     p = np.asarray(p, np.float64)

@@ -1089,6 +1089,21 @@ def effective_inflow_layer(pressure, temperature, dewpoint, vert_dim="model_leve
     return lay.dataset(out)
 
 
+def _vertical_pressure(pressure, lay):
+    """A shared 1-D pressure axis [L] reshaped to broadcast along the layout's vertical axis.  The pointwise functions
+    broadcast like NumPy, which would align [L] with the last axis of the fields instead; anything else (per-point
+    pressure, xarray inputs, which align by dimension name) is returned as it is."""
+    if lay.is_xr or len(lay.shape) < 2 or lay.vert_axis is None:
+        return pressure
+    if not isinstance(pressure, torch.Tensor):
+        pressure = np.asarray(pressure)
+    if pressure.ndim != 1 or pressure.shape[0] != lay.L:
+        return pressure
+    shape = [1] * len(lay.shape)
+    shape[lay.vert_axis] = lay.L
+    return pressure.reshape(shape)
+
+
 def melting_level_height(pressure, temperature, dewpoint, height, fast=True, vert_dim="model_level_number",
                          vert_axis=0, device=None):
     """PF:2162-2191: lowest height at which the wet-bulb temperature (1/3 rule with fast=True, Normand's
@@ -1096,7 +1111,8 @@ def melting_level_height(pressure, temperature, dewpoint, height, fast=True, ver
     if fast:
         wb = wet_bulb_temperature_fast(temperature, dewpoint)
     else:
-        wb = wet_bulb_temperature(pressure, temperature, dewpoint, vert_dim=vert_dim, device=device)
+        p = _vertical_pressure(pressure, _Layout(temperature, vert_dim, vert_axis))
+        wb = wet_bulb_temperature(p, temperature, dewpoint, vert_dim=vert_dim, device=device)
     return freezing_level_height(wb, height, vert_dim=vert_dim, vert_axis=vert_axis, device=device), wb
 
 
@@ -1190,7 +1206,8 @@ def storm_proxies(dat, device=None):
 
 def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat, downdraft=False, effective=False):
     p, t = dat["pressure"], dat["temperature"]
-    td = dewpoint_from_specific_humidity(p, t, dat["specific_humidity"], metpy_compat, device=device)
+    td = dewpoint_from_specific_humidity(_vertical_pressure(p, _Layout(t, vert_dim, vert_axis)), t,
+                                         dat["specific_humidity"], metpy_compat, device=device)
     try:
         dat["dewpoint"] = td                                        # the reference adds it to the caller's Dataset
     except Exception:
