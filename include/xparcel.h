@@ -22,12 +22,17 @@
  *  - mem = XP_MEM_DEVICE: pointers are device pointers on the context's device and the
  *    call is asynchronous on `stream` (a cudaStream_t passed as void*; NULL = default).
  *    mem = XP_MEM_HOST: pointers are host pointers; the library streams column blocks
- *    through three device slots on three streams (H2D, kernel, D2H of different blocks
- *    overlap) and returns when the outputs are complete.  The copies are issued straight
- *    from / to the caller's buffers: page-locked (pinned, cudaHostAlloc / cudaHostRegister)
- *    buffers copy asynchronously at PCIe speed; pageable buffers work too, but the driver
- *    then stages every copy through its own bounce buffers, synchronously (measured:
- *    bench.py extras.e2e_pageable vs e2e).
+ *    (XP_HOST_BLOCK_MB per block, default 192) through three device slots on three streams
+ *    (H2D, kernel, D2H of different blocks overlap) and returns when the outputs are
+ *    complete.  Page-locked (pinned, cudaHostAlloc / cudaHostRegister) buffers are copied
+ *    asynchronously, straight from / to the caller's memory.  Pageable buffers (what NumPy
+ *    arrays are) are staged by the library: XP_HOST_THREADS host threads copy each block
+ *    between the caller's arrays and a page-locked mirror of its slot, the DMA runs from /
+ *    to the mirror, and the outputs of a block are copied out of the mirror when its slot
+ *    is reused or the call drains.  Inputs are staged when any of them is pageable;
+ *    outputs when the first requested one of cape, cin, lcl/lfc/el/parcel pressure,
+ *    level_shift, profile pressure / temperature is -- otherwise they are copied directly.
+ *    Column blocks may be slices of wider arrays (level stride > n_columns).
  *  - Reference `assert`s that depend on data (PF:131 'Vertical pressures are not unique',
  *    PF:1149 'Top temperature is NaN.') are reported through xp_take_flags().
  */
@@ -399,7 +404,8 @@ xp_status xp_storm_proxies(xp_context *ctx, const xp_proxy_inputs *in, int64_t n
 uint64_t xp_launch_count(const xp_context *ctx);
 /* Columns of the most recent xp_cape_cin/xp_suite call that took the float32 fast path and were
  * recomputed by the float64 exact kernel because a decision was within the float32 error margin
- * (-1 if that call did not use the fast path).  Synchronises the call's stream. */
+ * (-1 if that call did not use the fast path).  Synchronises the call's stream.  After a call with
+ * mem = XP_MEM_HOST: the sum over all its column blocks (-1 if no block took the fast path). */
 xp_status xp_last_exact_count(xp_context *ctx, int64_t *out_count);
 /* Device time (ms) of the most recent xp_cape_cin/xp_suite kernel launch with
  * mem = XP_MEM_DEVICE, measured with CUDA events on the launch stream; syncs the stream. */

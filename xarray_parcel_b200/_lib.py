@@ -313,7 +313,9 @@ class Context:
 
     def last_exact_count(self):
         """Columns of the last call that the float32 fast path handed to the exact kernel (-1: the
-        call did not use the fast path)."""
+        call did not use the fast path).  For a call on CPU tensors (host memory, staged through the device in
+        column blocks of XP_HOST_BLOCK_MB on XP_HOST_THREADS copy threads): the sum over all its blocks (-1: no
+        block took the fast path)."""
         n = c_int64(0)
         self._check(self.lib.xp_last_exact_count(self.handle, ctypes.byref(n)), "xp_last_exact_count")
         return n.value

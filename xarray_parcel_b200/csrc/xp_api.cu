@@ -46,6 +46,12 @@ struct xp_context {
     std::map<cudaStream_t, Scratch> scratch;
     cudaStream_t last_fast_stream = nullptr;
     bool last_was_fast = false;
+    // XP_MEM_HOST calls: the fix-up list count of every block, copied on the block's slot stream into a page-locked
+    // array (one entry per block, read once the call has drained), and the call's total (-1: no block was fast)
+    uint32_t *block_count_pin = nullptr;
+    size_t block_count_cap = 0;
+    bool last_was_host = false;
+    int64_t last_host_exact = -1;
     int sm_count = 148;
     // experiment knobs, read from the environment once in xp_create (never in the launch path)
     int vote_mask = 3;
@@ -280,6 +286,7 @@ xp_status run_host(xp_context *ctx, const xp_columns *cols, int kind_mask,
     const size_t es = elt_size(cols->dtype);
     const int L = cols->n_levels;
     const int64_t N = cols->n_columns;
+    ctx->last_host_exact = -1;
     if (N == 0) return XP_OK;
     // per-column device bytes: inputs + every requested output
     size_t per_col = (size_t)(cols->pressure_is_1d ? 2 : 3) * L * es;
@@ -338,6 +345,16 @@ xp_status run_host(xp_context *ctx, const xp_columns *cols, int kind_mask,
         for (int s = 0; s < xp_context::kSlots; ++s) XP_CUDA(ctx, cudaHostAlloc(&ctx->slot_pin[s], need, cudaHostAllocDefault));
         ctx->slot_pin_bytes = need;
     }
+    // 4 bytes per block of >= 1024 columns: at most 1/2048 of the call's input bytes
+    const size_t n_blocks = (size_t)((N + C - 1) / C);
+    if (n_blocks > ctx->block_count_cap) {
+        if (ctx->block_count_pin) { cudaFreeHost(ctx->block_count_pin); ctx->block_count_pin = nullptr; }
+        ctx->block_count_cap = 0;
+        const size_t cap = std::max<size_t>(64, n_blocks);
+        XP_CUDA(ctx, cudaHostAlloc((void **)&ctx->block_count_pin, cap * sizeof(uint32_t), cudaHostAllocDefault));
+        ctx->block_count_cap = cap;
+    }
+    std::vector<char> block_fast(n_blocks, 0);
     // outputs of a block that wait in the page-locked mirror of its slot until the slot's stream has drained
     std::vector<RowCopy> pending_out[xp_context::kSlots];
     auto retire = [&](int s) -> xp_status {
@@ -361,7 +378,8 @@ xp_status run_host(xp_context *ctx, const xp_columns *cols, int kind_mask,
     const char *hp = (const char *)cols->pressure, *ht = (const char *)cols->temperature,
                *htd = (const char *)cols->dewpoint;
     int slot = 0;
-    for (int64_t c0 = 0; c0 < N; c0 += C, slot = (slot + 1) % xp_context::kSlots) {
+    int64_t blk = 0;
+    for (int64_t c0 = 0; c0 < N; c0 += C, slot = (slot + 1) % xp_context::kSlots, ++blk) {
         const int64_t n = std::min<int64_t>(C, N - c0);
         cudaStream_t st = ctx->slot_stream[slot];
         char *base = (char *)ctx->slot_buf[slot];
@@ -467,6 +485,12 @@ xp_status run_host(xp_context *ctx, const xp_columns *cols, int kind_mask,
                             ? run_device<float>(ctx, &dc, kind_mask, douts, &dex, o, st, false)
                             : run_device<double>(ctx, &dc, kind_mask, douts, &dex, o, st, false);
         if (stt != XP_OK) return stt;
+        if (ctx->last_was_fast) {
+            // the block's hand-over count, before the next fast block on this stream resets it in the scratch
+            XP_CUDA(ctx, cudaMemcpyAsync(ctx->block_count_pin + blk, fast_list_count_ptr(ctx->scratch[st].ptr),
+                                         sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+            block_fast[blk] = 1;
+        }
         for (const Copy &c : copies) {
             if (stage_out) {
                 // device -> page-locked mirror now; mirror -> caller when the slot is retired
@@ -486,6 +510,8 @@ xp_status run_host(xp_context *ctx, const xp_columns *cols, int kind_mask,
         XP_CUDA(ctx, cudaStreamSynchronize(ctx->slot_stream[s]));
         if (!pending_out[s].empty()) { parallel_copy(pending_out[s], ctx->host_threads); pending_out[s].clear(); }
     }
+    for (size_t b = 0; b < n_blocks; ++b)
+        if (block_fast[b]) ctx->last_host_exact = std::max<int64_t>(ctx->last_host_exact, 0) + ctx->block_count_pin[b];
     return XP_OK;
 }
 
@@ -501,6 +527,7 @@ xp_status run_any(xp_context *ctx, const xp_columns *cols, int kind_mask,
     if (cols->n_columns == 0) return XP_OK;
     DeviceGuard guard(ctx->device);
     const Opts o = to_opts(ctx, opts);
+    ctx->last_was_host = cols->mem == XP_MEM_HOST;
     if (cols->mem == XP_MEM_HOST) return run_host(ctx, cols, kind_mask, outs, ex, o);
     if (cols->dtype == XP_F32)
         return run_device<float>(ctx, cols, kind_mask, outs, ex, o, (cudaStream_t)stream, true);
@@ -576,6 +603,7 @@ void xp_destroy(xp_context *ctx) {
             if (ctx->slot_pin[s]) cudaFreeHost(ctx->slot_pin[s]);
             if (ctx->slot_stream[s]) cudaStreamDestroy(ctx->slot_stream[s]);
         }
+        if (ctx->block_count_pin) cudaFreeHost(ctx->block_count_pin);
         for (auto &kv : ctx->scratch) cudaFree(kv.second.ptr);
         if (ctx->ev0) cudaEventDestroy(ctx->ev0);
         if (ctx->ev1) cudaEventDestroy(ctx->ev1);
@@ -1217,6 +1245,7 @@ xp_status xp_last_exact_count(xp_context *ctx, int64_t *out_count) {
     if (!ctx || !out_count) return XP_ERR_INVALID_ARGUMENT;
     std::lock_guard<std::mutex> lock(ctx->mu);
     *out_count = -1;
+    if (ctx->last_was_host) { *out_count = ctx->last_host_exact; return XP_OK; }    // every block of the call
     if (!ctx->last_was_fast) return XP_OK;
     DeviceGuard guard(ctx->device);
     auto it = ctx->scratch.find(ctx->last_fast_stream);

@@ -813,12 +813,16 @@ int launch_suite_fast_f64(const ColsArg<double> &cols, const Tables &tb, const O
     return 4;
 }
 
+const uint32_t *fast_list_count_ptr(const void *scratch) {
+    const unsigned char *base = static_cast<const unsigned char *>(scratch);
+    const size_t off = ((sizeof(Prep) + 255) & ~(size_t)255) + (size_t)fast::kMaxLevels * fast::kNI * sizeof(Coef);
+    return reinterpret_cast<const uint32_t *>(base + off) + 3;
+}
+
 // number of list entries of the last fast launch (debug/metrics; synchronous copy)
 uint32_t fast_last_list_count(void *scratch, cudaStream_t stream) {
-    unsigned char *base = static_cast<unsigned char *>(scratch);
-    size_t off = ((sizeof(Prep) + 255) & ~(size_t)255) + (size_t)fast::kMaxLevels * fast::kNI * sizeof(Coef);
     uint32_t v = 0;
-    cudaMemcpyAsync(&v, base + off + 3 * sizeof(uint32_t), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream);
+    cudaMemcpyAsync(&v, fast_list_count_ptr(scratch), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream);
     cudaStreamSynchronize(stream);
     return v;
 }

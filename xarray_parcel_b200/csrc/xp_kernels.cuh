@@ -142,6 +142,8 @@ int launch_suite_fast(const ColsArg<float> &cols, const Tables &tb, const Opts &
                       const OutArg<float> *outs, void *scratch, uint32_t *flags, int sm_count,
                       cudaStream_t stream);
 uint32_t fast_last_list_count(void *scratch, cudaStream_t stream);
+// device address of that count (columns with at least one list entry) inside `scratch`
+const uint32_t *fast_list_count_ptr(const void *scratch);
 // The same fast path for float64 columns and outputs on a shared pressure axis with the reference's default options
 // (the v7 sweep: float32 per level, float64 parcels; the fix-up list runs on the float64 columns).  Returns the
 // number of launches, or -2 when the call does not qualify (the caller then runs the float64 exact kernel).
