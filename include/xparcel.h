@@ -380,6 +380,58 @@ typedef struct xp_effective_out {
 } xp_effective_out;
 xp_status xp_effective_inflow_layer(xp_context *ctx, const xp_columns *cols, const xp_options *opts, double min_cape,
                                     double min_cin, const xp_effective_out *out, void *stream);
+/* xp_storm_kinematics: Bunkers storm motion, storm-relative helicity (SRH) and bulk wind difference (BWD) per column,
+ * device memory only.  Contract (DESIGN.md section 3.14), float64 arithmetic:
+ *  - wind profile: the surface point (z = 0, surface_u, surface_v), then, in level order, every level whose height z
+ *    (m above the surface), u and v are all non-NaN and whose z > 0; a NaN surface wind or kept heights that do not
+ *    increase strictly make every output of the column NaN; V(z) is the profile interpolated linearly in height;
+ *  - layer [a, b], a bound below 0 taken as 0: the points a, the profile points strictly inside (a, b), and b; NaN if a
+ *    or b is NaN, b < a or b lies above the highest profile point read.  Mean wind = trapezoid(V, z) / (b - a); SRH(c) =
+ *    sum (u_{i+1} - c_u)(v_i - c_v) - (u_i - c_u)(v_{i+1} - c_v) over consecutive layer points [m2/s2] (0 for a == b);
+ *    BWD = V(b) - V(a);
+ *  - Bunkers (Bunkers et al. 2000): M = mean wind over [0, 6000], S = mean over [5500, 6000] - mean over [0, 500],
+ *    right / left = M +- 7.5 (S_v, -S_u) / |S|, NaN if |S| == 0 or a layer is NaN; SRH uses the `mover`'s motion
+ *    (+1 right, -1 left) and is NaN where it is;
+ *  - a column is read up to the first profile point at or above the highest bound the call needs (6000 m for the motion
+ *    and any SRH) and no further; the strictly-increasing check covers those points.
+ * Outputs, in the input dtype, [n_columns] each, any may be NULL: the motion and mean wind; srh[j], SRH over
+ * [0, depths[j]] for j < n_depths; srh_layer over [srh_bottom, srh_top]; bwd_u / bwd_v / bwd_magnitude over
+ * [bwd_bottom, bwd_top].  XP_ERR_INVALID_ARGUMENT for a NULL wind input, `in` or `out`, n_levels < 1, a level stride
+ * below n_columns, n_depths outside 0..4, a depth that is not positive and finite, a mover other than +-1, a layer
+ * bottom without its top (or the reverse), srh[j] for j >= n_depths, or a layer output without its bounds. */
+typedef struct xp_wind_columns {
+    const void *height, *wind_u, *wind_v;   /* [n_levels][n_columns], level stride level_stride; m AGL, m/s */
+    const void *surface_u, *surface_v;      /* [n_columns] */
+    int64_t n_columns;
+    int32_t n_levels;
+    int32_t dtype;                          /* xp_dtype */
+    int64_t level_stride;
+} xp_wind_columns;
+typedef struct xp_kinematics_in {
+    int32_t mover;                          /* +1 right mover, -1 left mover */
+    int32_t n_depths;                       /* 0..4 */
+    double depths[4];                       /* m AGL, positive and finite */
+    const void *srh_bottom, *srh_top;       /* [n_columns] m AGL, or both NULL */
+    const void *bwd_bottom, *bwd_top;       /* [n_columns] m AGL, or both NULL */
+} xp_kinematics_in;
+typedef struct xp_kinematics_out {
+    void *right_u, *right_v, *left_u, *left_v, *mean_u, *mean_v;    /* m/s */
+    void *srh[4];                                                   /* m2/s2 */
+    void *srh_layer;                                                /* m2/s2 */
+    void *bwd_u, *bwd_v, *bwd_magnitude;                            /* m/s */
+} xp_kinematics_out;
+xp_status xp_storm_kinematics(xp_context *ctx, const xp_wind_columns *cols, const xp_kinematics_in *in,
+                              const xp_kinematics_out *out, void *stream);
+/* xp_supercell_tornado_parameters: pointwise, device memory only, float64 arithmetic, NaN in gives NaN out.
+ *  scp = (mucape / 1000) (esrh / 50) t_b with t_b = 0 if ebwd < 10, 1 if ebwd > 20, else ebwd / 20 (SHARPpy scp);
+ *  stp = max(0, (mlcape / 1500) (esrh / 150) t_b t_lcl t_cin) (np.maximum: NaN stays NaN) with t_b = 0 if ebwd < 12.5,
+ *  1.5 if ebwd > 30, else ebwd / 20; t_lcl = 1 if lcl_height < 1000, 0 if > 2000, else (2000 - lcl_height) / 1000;
+ *  t_cin = 1 if mlcin > -50, 0 if < -200, else (mlcin + 200) / 150 (SHARPpy stp_cin).
+ * Units J/kg, m2/s2, m/s, m AGL.  scp or stp may be NULL; the inputs of a requested output must not be
+ * (XP_ERR_INVALID_ARGUMENT). */
+xp_status xp_supercell_tornado_parameters(xp_context *ctx, const void *mucape, const void *esrh, const void *ebwd,
+                                          const void *mlcape, const void *mlcin, const void *lcl_height, int64_t n,
+                                          int32_t dtype, void *scp, void *stp, void *stream);
 /* significant_hail_parameter (PF:2261-2306): units as the reference's arguments (mixing ratio kg/kg,
  * lapse K/km negative for decreasing temperature, temp_500 K, shear m/s, flh m). */
 xp_status xp_significant_hail_parameter(xp_context *ctx, const void *mucape, const void *mixing_ratio,

@@ -14,4 +14,4 @@ export XP_HOSTSIM_SANITIZE=1
 export ASAN_OPTIONS=detect_leaks=0:abort_on_error=1
 LD_PRELOAD="$(gcc -print-file-name=libasan.so):$(gcc -print-file-name=libubsan.so)" \
     python -m pytest tests/test_fast_hostsim.py tests/test_hostsim_vs_oracle.py tests/test_layers_hostsim.py \
-    tests/test_levels_hostsim.py tests/test_specific_humidity_input.py -q -m "not gpu" -p no:cacheprovider "$@"
+    tests/test_levels_hostsim.py tests/test_specific_humidity_input.py tests/test_kinematics_hostsim.py -q -m "not gpu" -p no:cacheprovider "$@"

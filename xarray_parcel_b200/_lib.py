@@ -67,7 +67,7 @@ EXPORTS = ["xp_version", "xp_create", "xp_destroy", "xp_last_error", "xp_take_fl
            "xp_significant_hail_parameter", "xp_storm_proxies", "xp_mixed_layer", "xp_mixed_parcel",
            "xp_layer_bounds", "xp_insert_level", "xp_shift_out_nans", "xp_trapz", "xp_valid_data",
            "xp_find_intersections", "xp_interp1d", "xp_trap_around_zeros", "xp_downdraft_cape",
-           "xp_effective_inflow_layer"]
+           "xp_effective_inflow_layer", "xp_storm_kinematics", "xp_supercell_tornado_parameters"]
 
 PROXY_INPUTS = ["mixed_100_cape", "mixed_50_cape", "mu_cape", "shear_magnitude", "mixed_100_lifted_index",
                 "mixed_100_dci", "positive_shear", "mixed_50_cin", "mixed_100_cin", "lapse_rate_700_500",
@@ -113,6 +113,31 @@ EFFECTIVE_LEVEL_FIELDS = ["level_parcel_cape", "level_parcel_cin"]
 class XpEffectiveOut(ctypes.Structure):
     _fields_ = [("base_pressure", c_void_p), ("top_pressure", c_void_p), ("level_cape", c_void_p),
                 ("level_cin", c_void_p), ("level_out_stride", c_int64)]
+
+
+MOTION_FIELDS = ["bunkers_right_u", "bunkers_right_v", "bunkers_left_u", "bunkers_left_v", "mean_wind_u",
+                 "mean_wind_v"]
+BWD_FIELDS = ["bulk_wind_difference_u", "bulk_wind_difference_v", "bulk_wind_difference"]
+COMPOSITE_FIELDS = ["supercell_composite_parameter", "significant_tornado_parameter"]
+EFFECTIVE_PARAMETER_FIELDS = ["effective_srh", "effective_bulk_wind_difference"] + COMPOSITE_FIELDS
+MOVERS = {"right": 1, "left": -1}
+
+
+class XpWindColumns(ctypes.Structure):
+    _fields_ = [("height", c_void_p), ("wind_u", c_void_p), ("wind_v", c_void_p), ("surface_u", c_void_p),
+                ("surface_v", c_void_p), ("n_columns", c_int64), ("n_levels", c_int32), ("dtype", c_int32),
+                ("level_stride", c_int64)]
+
+
+class XpKinematicsIn(ctypes.Structure):
+    _fields_ = [("mover", c_int32), ("n_depths", c_int32), ("depths", c_double * 4), ("srh_bottom", c_void_p),
+                ("srh_top", c_void_p), ("bwd_bottom", c_void_p), ("bwd_top", c_void_p)]
+
+
+class XpKinematicsOut(ctypes.Structure):
+    _fields_ = ([(n, c_void_p) for n in ("right_u", "right_v", "left_u", "left_v", "mean_u", "mean_v")] +
+                [("srh", c_void_p * 4), ("srh_layer", c_void_p)] +
+                [(n, c_void_p) for n in ("bwd_u", "bwd_v", "bwd_magnitude")])
 
 
 class XpProxyInputs(ctypes.Structure):
@@ -220,6 +245,10 @@ def load_library():
                                           c_int64, c_int32, c_int32, ctypes.POINTER(XpDowndraftOut), c_void_p]
         lib.xp_effective_inflow_layer.argtypes = [c_void_p, ctypes.POINTER(XpColumns), ctypes.POINTER(XpOptions),
                                                   c_double, c_double, ctypes.POINTER(XpEffectiveOut), c_void_p]
+        lib.xp_storm_kinematics.argtypes = [c_void_p, ctypes.POINTER(XpWindColumns), ctypes.POINTER(XpKinematicsIn),
+                                            ctypes.POINTER(XpKinematicsOut), c_void_p]
+        lib.xp_supercell_tornado_parameters.argtypes = [c_void_p] + [c_void_p] * 6 + [c_int64, c_int32, c_void_p,
+                                                                                      c_void_p, c_void_p]
         lib.xp_launch_count.argtypes = [c_void_p]
         lib.xp_launch_count.restype = ctypes.c_uint64
         lib.xp_last_kernel_ms.argtypes = [c_void_p, ctypes.POINTER(ctypes.c_float)]
@@ -670,6 +699,79 @@ class Context:
                                                 float(min_cin), ctypes.byref(o), self._stream())
         self._check(st, "xp_effective_inflow_layer")
         return res
+
+    def storm_kinematics(self, height, wind_u, wind_v, surface_u, surface_v, mover="right", depths=(),
+                         srh_layer=None, bwd_layer=None, outputs=None):
+        """Storm kinematics (xp_storm_kinematics) of the device wind columns ``wind_u`` / ``wind_v`` [L, N] on
+        ``height`` [L, N] (m above the surface) with the surface wind [N].  Returns a dict of [N] tensors: the
+        MOTION_FIELDS, 'srh_0_<d>m' for each of up to 4 ``depths`` [m], with ``srh_layer=(bottom, top)`` ([N] m AGL)
+        'srh_layer' and with ``bwd_layer=(bottom, top)`` the BWD_FIELDS.  ``mover``: 'right' or 'left' (the motion
+        SRH is taken relative to).  ``outputs`` (a subset of those names) leaves the others uncomputed."""
+        L, N = wind_u.shape
+        dt = wind_u.dtype
+        z, u, v = [x.to(dt) for x in (height, wind_u, wind_v)]
+        if z.shape != (L, N) or v.shape != (L, N):
+            raise ValueError("height / wind_u / wind_v must be [n_levels, n_columns]")
+        if not (N <= 1 or all(x.stride(1) == 1 for x in (z, u, v))) or len({x.stride(0) for x in (z, u, v)}) > 1 \
+                or (L > 1 and u.stride(0) < N):
+            z, u, v = z.contiguous(), u.contiguous(), v.contiguous()
+        su, sv = [x.to(dt).expand(N).contiguous() for x in (surface_u, surface_v)]
+        depths = [float(d) for d in depths]
+        srh_names = [f"srh_0_{d:g}m" for d in depths]
+        names = list(MOTION_FIELDS) + srh_names + (["srh_layer"] if srh_layer is not None else []) + \
+            (list(BWD_FIELDS) if bwd_layer is not None else [])
+        if outputs is not None:
+            names = [n for n in names if n in outputs]
+        res = {n: torch.empty((N,), dtype=dt, device=u.device) for n in names}
+        ptr = lambda n: res[n].data_ptr() if n in res else None          # noqa: E731
+        keep = []
+
+        def bounds(layer):
+            if layer is None:
+                return None, None
+            b = [x.to(dt).expand(N).contiguous() for x in layer]
+            keep.extend(b)
+            return b[0].data_ptr(), b[1].data_ptr()
+
+        if len(depths) > 4:
+            raise ValueError("at most 4 SRH depths per call")
+        d4 = (c_double * 4)(*(depths + [0.0] * (4 - len(depths))))
+        sb, st = bounds(srh_layer)
+        bb, bt = bounds(bwd_layer)
+        kin = XpKinematicsIn(MOVERS[mover], len(depths), d4, sb, st, bb, bt)
+        o = XpKinematicsOut(*[ptr(n) for n in MOTION_FIELDS], (c_void_p * 4)(*[ptr(n) for n in srh_names]),
+                            ptr("srh_layer"), *[ptr(n) for n in BWD_FIELDS])
+        cols = XpWindColumns(z.data_ptr(), u.data_ptr(), v.data_ptr(), su.data_ptr(), sv.data_ptr(), N, L,
+                             _dtype_code(u), u.stride(0) if L > 1 else N)
+        st_ = self.lib.xp_storm_kinematics(self.handle, ctypes.byref(cols), ctypes.byref(kin), ctypes.byref(o),
+                                           self._stream())
+        self._check(st_, "xp_storm_kinematics")
+        return res
+
+    def supercell_tornado_parameters(self, mucape, esrh, ebwd, mlcape, mlcin, lcl_height, outputs=COMPOSITE_FIELDS):
+        """Supercell composite and significant tornado parameters (xp_supercell_tornado_parameters) of broadcast
+        device tensors.  Returns a dict of the requested COMPOSITE_FIELDS; the inputs only the other output needs may
+        be None."""
+        dt = esrh.dtype
+        ins = [mucape, esrh, ebwd, mlcape, mlcin, lcl_height]
+        given = [x for x in ins if x is not None]
+        bc = iter([x.to(dt).contiguous() for x in torch.broadcast_tensors(*given)])
+        xs = [next(bc) if x is not None else None for x in ins]
+        like = xs[1]
+        res = {n: torch.empty_like(like) for n in COMPOSITE_FIELDS if n in outputs}
+        ptr = [res[n].data_ptr() if n in res else None for n in COMPOSITE_FIELDS]
+        st = self.lib.xp_supercell_tornado_parameters(self.handle, *[x.data_ptr() if x is not None else None for x in xs],
+                                                      like.numel(), _dtype_code(like), ptr[0], ptr[1], self._stream())
+        self._check(st, "xp_supercell_tornado_parameters")
+        return res
+
+    def supercell_composite_parameter(self, mucape, esrh, ebwd):
+        return self.supercell_tornado_parameters(mucape, esrh, ebwd, None, None, None,
+                                                 outputs=COMPOSITE_FIELDS[:1])[COMPOSITE_FIELDS[0]]
+
+    def significant_tornado_parameter(self, mlcape, esrh, ebwd, lcl_height, mlcin):
+        return self.supercell_tornado_parameters(None, esrh, ebwd, mlcape, mlcin, lcl_height,
+                                                 outputs=COMPOSITE_FIELDS[1:])[COMPOSITE_FIELDS[1]]
     # ---- level primitives (xp_levels.cu) ---------------------------------------------------------------
     @staticmethod
     def _ptrs(tensors):

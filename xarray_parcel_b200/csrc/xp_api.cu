@@ -2,6 +2,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -14,6 +15,7 @@
 
 #include "../../include/xparcel.h"
 #include "xp_kernels.cuh"
+#include "xp_kinematics.cuh"
 
 using namespace xp;
 
@@ -1196,6 +1198,77 @@ xp_status xp_effective_inflow_layer(xp_context *ctx, const xp_columns *cols, con
     if (rc < 0) return fail(ctx, XP_ERR_INVALID_ARGUMENT, "effective_inflow_layer: too many levels on a shared axis");
     ctx->launches += 2;
     return check_cuda(ctx, cudaGetLastError(), "effective_inflow_layer kernel launch");
+}
+
+// Storm kinematics, contract in include/xparcel.h and xp_kinematics.cuh (DESIGN.md section 3.14).
+xp_status xp_storm_kinematics(xp_context *ctx, const xp_wind_columns *cols, const xp_kinematics_in *in,
+                              const xp_kinematics_out *out, void *stream) {
+    if (!ctx) return XP_ERR_INVALID_ARGUMENT;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if (!cols || !in || !out || !cols->height || !cols->wind_u || !cols->wind_v || !cols->surface_u ||
+        !cols->surface_v)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "storm_kinematics: NULL input");
+    if (cols->n_levels < 1 || cols->n_columns < 0)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "storm_kinematics: n_levels < 1 or n_columns < 0");
+    if (cols->n_levels > 1 && cols->level_stride < cols->n_columns)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "storm_kinematics: level stride smaller than a level");
+    if (cols->dtype != XP_F32 && cols->dtype != XP_F64)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "dtype must be XP_F32 or XP_F64");
+    if (in->mover != 1 && in->mover != -1)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "storm_kinematics: mover must be +1 (right) or -1 (left)");
+    if (in->n_depths < 0 || in->n_depths > kMaxSrhDepths)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "storm_kinematics: n_depths must be 0..4");
+    for (int j = 0; j < in->n_depths; ++j)
+        if (!(in->depths[j] > 0.0) || !std::isfinite(in->depths[j]))
+            return fail(ctx, XP_ERR_INVALID_ARGUMENT, "storm_kinematics: depths must be positive and finite");
+    for (int j = in->n_depths; j < kMaxSrhDepths; ++j)
+        if (out->srh[j]) return fail(ctx, XP_ERR_INVALID_ARGUMENT, "storm_kinematics: srh[j] with j >= n_depths");
+    if (!in->srh_bottom != !in->srh_top || !in->bwd_bottom != !in->bwd_top)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "storm_kinematics: a layer bottom without its top");
+    if ((out->srh_layer && !in->srh_bottom) || ((out->bwd_u || out->bwd_v || out->bwd_magnitude) && !in->bwd_bottom))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "storm_kinematics: a layer output without its layer");
+    if (cols->n_columns == 0) return XP_OK;
+    void *motion[6] = {out->right_u, out->right_v, out->left_u, out->left_v, out->mean_u, out->mean_v};
+    void *bwd[3] = {out->bwd_u, out->bwd_v, out->bwd_magnitude};
+    KinematicsRequest rq;
+    rq.motion = false;
+    for (void *m : motion) rq.motion = rq.motion || m;
+    rq.n_depths = 0;
+    for (int j = 0; j < kMaxSrhDepths; ++j) {
+        rq.depth[j] = j < in->n_depths ? in->depths[j] : 0.0;
+        if (j < in->n_depths && out->srh[j]) rq.n_depths = j + 1;     // trailing unrequested depths are not computed
+    }
+    rq.srh_layer = out->srh_layer != nullptr;
+    rq.bwd_layer = bwd[0] || bwd[1] || bwd[2];
+    rq.mover = (double)in->mover;
+    if (!rq.motion && rq.n_depths == 0 && !rq.srh_layer && !rq.bwd_layer) return XP_OK;
+    DeviceGuard guard(ctx->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t ls = cols->n_levels > 1 ? cols->level_stride : cols->n_columns;
+    XP_DISPATCH(cols->dtype,
+                launch_storm_kinematics<float>((const float *)cols->height, (const float *)cols->wind_u, (const float *)cols->wind_v, (const float *)cols->surface_u, (const float *)cols->surface_v, ls, cols->n_levels, cols->n_columns, rq, (const float *)in->srh_bottom, (const float *)in->srh_top, (const float *)in->bwd_bottom, (const float *)in->bwd_top, (float *const *)motion, (float *const *)out->srh, (float *)out->srh_layer, (float *const *)bwd, st),
+                launch_storm_kinematics<double>((const double *)cols->height, (const double *)cols->wind_u, (const double *)cols->wind_v, (const double *)cols->surface_u, (const double *)cols->surface_v, ls, cols->n_levels, cols->n_columns, rq, (const double *)in->srh_bottom, (const double *)in->srh_top, (const double *)in->bwd_bottom, (const double *)in->bwd_top, (double *const *)motion, (double *const *)out->srh, (double *)out->srh_layer, (double *const *)bwd, st));
+    ctx->launches += 1;
+    return check_cuda(ctx, cudaGetLastError(), "storm_kinematics kernel launch");
+}
+
+xp_status xp_supercell_tornado_parameters(xp_context *ctx, const void *mucape, const void *esrh, const void *ebwd,
+                                          const void *mlcape, const void *mlcin, const void *lcl_height, int64_t n,
+                                          int32_t dtype, void *scp, void *stp, void *stream) {
+    if (!ctx) return XP_ERR_INVALID_ARGUMENT;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if (n < 0 || ((scp || stp) && (!esrh || !ebwd)) || (scp && !mucape) || (stp && (!mlcape || !mlcin || !lcl_height)))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad supercell_tornado_parameters arguments");
+    if (dtype != XP_F32 && dtype != XP_F64)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "dtype must be XP_F32 or XP_F64");
+    if (n == 0 || (!scp && !stp)) return XP_OK;
+    DeviceGuard guard(ctx->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    XP_DISPATCH(dtype,
+                launch_composite_parameters<float>((const float *)mucape, (const float *)esrh, (const float *)ebwd, (const float *)mlcape, (const float *)mlcin, (const float *)lcl_height, n, (float *)scp, (float *)stp, st),
+                launch_composite_parameters<double>((const double *)mucape, (const double *)esrh, (const double *)ebwd, (const double *)mlcape, (const double *)mlcin, (const double *)lcl_height, n, (double *)scp, (double *)stp, st));
+    ctx->launches += 1;
+    return check_cuda(ctx, cudaGetLastError(), "supercell_tornado_parameters kernel launch");
 }
 
 xp_status xp_significant_hail_parameter(xp_context *ctx, const void *mucape, const void *mixing_ratio,

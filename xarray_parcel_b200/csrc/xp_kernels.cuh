@@ -242,6 +242,20 @@ int launch_effective(const ColsArg<T> &cols, const Tables &tb, const Opts &o, do
                      T *base, T *top, T *lcape, T *lcin, int64_t lls, uint32_t *flags, void *scratch, int sm_count,
                      cudaStream_t stream);
 
+// Storm kinematics (xp_kinematics.cu, contract in xp_kinematics.cuh): motion6 = Bunkers right u / v, left u / v, mean
+// wind u / v; srh4 = SRH over the request's fixed depths; bwd3 = BWD u / v / magnitude; [N] each, any may be null.
+// sb / st (SRH layer) and bb / bt (BWD layer) are [N] or null.
+struct KinematicsRequest;
+template <typename T>
+void launch_storm_kinematics(const T *z, const T *u, const T *v, const T *su, const T *sv, int64_t ls, int L,
+                             int64_t n, const KinematicsRequest &rq, const T *sb, const T *st, const T *bb,
+                             const T *bt, T *const *motion6, T *const *srh4, T *srh_layer, T *const *bwd3,
+                             cudaStream_t stream);
+// Supercell composite and significant tornado parameters (xp_kinematics.cuh), pointwise over n; scp / stp may be null.
+template <typename T>
+void launch_composite_parameters(const T *mucape, const T *esrh, const T *ebwd, const T *mlcape, const T *mlcin,
+                                 const T *lcl_h, int64_t n, T *scp, T *stp, cudaStream_t stream);
+
 // Table builder (xp_tables.cu): fills index_grid (uint16 [kNP][kNT]) and curves (float
 // [kNAdiabats][kNP] ascending pressure).  `scratch_u32` must hold kNP*kNT uint32.
 void launch_build_tables(uint16_t *index_grid, float *curves, uint32_t *scratch_u32,

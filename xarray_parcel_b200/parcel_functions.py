@@ -37,7 +37,8 @@ __all__ = ["load_moist_adiabat_lookups", "lookup_tables_loaded", "moist_adiabat_
            "deep_convective_index", "isobar_temperature", "lapse_rate", "freezing_level_height",
            "melting_level_height", "wet_bulb_temperature_fast", "wind_shear",
            "dewpoint_from_specific_humidity", "conv_properties", "min_conv_properties", "downdraft_cape",
-           "effective_inflow_layer"]
+           "effective_inflow_layer", "bunkers_storm_motion", "storm_relative_helicity", "effective_layer_parameters",
+           "supercell_composite_parameter", "significant_tornado_parameter"]
 
 KAPPA = 0.28571428571428564       # metpy.constants.kappa (PF:313)
 
@@ -67,6 +68,17 @@ _ATTRS = {
     "effective_inflow_top": {"long_name": "Effective inflow layer top pressure", "units": "hPa"},
     "level_parcel_cape": {"long_name": "CAPE of the parcel lifted from each level", "units": "J kg$^{-1}$"},
     "level_parcel_cin": {"long_name": "CIN of the parcel lifted from each level", "units": "J kg$^{-1}$"},
+    "bunkers_right_u": {"long_name": "Bunkers right-mover storm motion, eastward", "units": "m s$^{-1}$"},
+    "bunkers_right_v": {"long_name": "Bunkers right-mover storm motion, northward", "units": "m s$^{-1}$"},
+    "bunkers_left_u": {"long_name": "Bunkers left-mover storm motion, eastward", "units": "m s$^{-1}$"},
+    "bunkers_left_v": {"long_name": "Bunkers left-mover storm motion, northward", "units": "m s$^{-1}$"},
+    "mean_wind_u": {"long_name": "0-6 km mean wind, eastward", "units": "m s$^{-1}$"},
+    "mean_wind_v": {"long_name": "0-6 km mean wind, northward", "units": "m s$^{-1}$"},
+    "effective_srh": {"long_name": "Effective storm-relative helicity", "units": "m$^{2}$ s$^{-2}$"},
+    "effective_bulk_wind_difference": {"long_name": "Effective bulk wind difference", "units": "m s$^{-1}$"},
+    "supercell_composite_parameter": {"long_name": "Supercell composite parameter", "units": "1"},
+    "significant_tornado_parameter": {"long_name": "Significant tornado parameter (effective layer, with CIN)",
+                                      "units": "1"},
 }
 
 
@@ -1089,6 +1101,131 @@ def effective_inflow_layer(pressure, temperature, dewpoint, vert_dim="model_leve
     return lay.dataset(out)
 
 
+def _wind_blocks(surface_wind_u, surface_wind_v, wind_u, wind_v, height, vert_dim, vert_axis, device):
+    ctx = _lib.get_context(device)
+    lay, dtype, on_gpu = _layout_of(wind_u, vert_dim, vert_axis)
+    dev = f"cuda:{ctx.device}"
+    u, v, h = [b.to(dev) for b in _blocks(lay, [wind_u, wind_v, height], dtype)]
+    su, sv = [lay.scalar_to_block(x, dtype).to(dev) for x in (surface_wind_u, surface_wind_v)]
+    return ctx, lay, on_gpu, h, u, v, su, sv
+
+
+def bunkers_storm_motion(surface_wind_u, surface_wind_v, wind_u, wind_v, height, vert_dim="model_level_number",
+                         vert_axis=0, device=None):
+    """Bunkers et al. (2000) storm motion by the internal-dynamics method, on the height-weighted 0-6 km mean wind
+    (``xp_storm_kinematics``, one CUDA thread per column; contract in DESIGN.md section 3.14).
+
+    The wind profile is the surface wind at 0 m followed by the levels with non-NaN height, u and v above the surface
+    (``height`` in m above the surface; levels at or below ground are dropped), linear in height.  The shear vector S is
+    the 5.5-6 km mean wind minus the 0-0.5 km mean wind; the right / left movers are the 0-6 km mean wind plus / minus
+    7.5 m/s normal to S.  Columns that do not reach 6 km, whose heights do not increase, with a NaN surface wind or
+    with S = 0 give NaN.  Returns a Dataset of bunkers_right_u/_v, bunkers_left_u/_v and mean_wind_u/_v [m/s]."""
+    ctx, lay, on_gpu, h, u, v, su, sv = _wind_blocks(surface_wind_u, surface_wind_v, wind_u, wind_v, height,
+                                                     vert_dim, vert_axis, device)
+    r = ctx.storm_kinematics(h, u, v, su, sv)
+    fix = (lambda x: x) if on_gpu else (lambda x: x.cpu())
+    return lay.dataset({k: lay.wrap_scalar(fix(r[k]), k) for k in _lib.MOTION_FIELDS})
+
+
+def storm_relative_helicity(surface_wind_u, surface_wind_v, wind_u, wind_v, height, depths=(1000, 3000),
+                            mover="right", vert_dim="model_level_number", vert_axis=0, device=None):
+    """Storm-relative helicity over 0-d m above the surface for each of up to 4 ``depths``, relative to the Bunkers
+    motion of the ``mover`` ('right' or 'left'; ``xp_storm_kinematics``, contract in DESIGN.md section 3.14).
+
+    SRH is MetPy's ``storm_relative_helicity`` total over the layer's points (its bottom, the profile levels inside,
+    its top, interpolated linearly in height), positive for a veering hodograph with the right mover.  NaN where the
+    Bunkers motion is NaN or the profile does not reach the depth.  Returns a Dataset of srh_0_<d>m [m2/s2]."""
+    ctx, lay, on_gpu, h, u, v, su, sv = _wind_blocks(surface_wind_u, surface_wind_v, wind_u, wind_v, height,
+                                                     vert_dim, vert_axis, device)
+    r = ctx.storm_kinematics(h, u, v, su, sv, mover=mover, depths=depths,
+                             outputs=[f"srh_0_{float(d):g}m" for d in depths])
+    fix = (lambda x: x) if on_gpu else (lambda x: x.cpu())
+    attrs = {k: {"long_name": f"Storm-relative helicity, {k[6:-1]} m ({mover} mover)", "units": "m$^{2}$ s$^{-2}$"}
+             for k in r}
+    ds = lay.dataset({k: lay.wrap_scalar(fix(r[k]), k) for k in r})
+    for k in r:
+        if isinstance(ds, Dataset):
+            ds.var_attrs[k] = attrs[k]
+        else:
+            ds[k].attrs.update(attrs[k])
+    return ds
+
+
+def supercell_composite_parameter(mucape, effective_srh, effective_bulk_wind_difference, device=None):
+    """Supercell composite parameter, SHARPpy's ``params.scp``: (mucape / 1000) (esrh / 50) t_b with t_b = 0 below
+    10 m/s of effective bulk wind difference, 1 above 20 m/s and ebwd / 20 between (``xp_supercell_tornado_parameters``,
+    pointwise; NaN in gives NaN out).  Units J/kg, m2/s2, m/s."""
+    return _pointwise("supercell_composite_parameter", [mucape, effective_srh, effective_bulk_wind_difference],
+                      name="supercell_composite_parameter", attrs=_ATTRS["supercell_composite_parameter"],
+                      device=device)
+
+
+def significant_tornado_parameter(mlcape, effective_srh, effective_bulk_wind_difference, lcl_height, mlcin,
+                                  device=None):
+    """Effective-layer significant tornado parameter with CIN, SHARPpy's ``params.stp_cin``: max(0, (mlcape / 1500)
+    (esrh / 150) t_b t_lcl t_cin) with t_b = 0 below 12.5 m/s of effective bulk wind difference, 1.5 above 30 m/s and
+    ebwd / 20 between; t_lcl = 1 below 1000 m of mixed-layer LCL height above the surface, 0 above 2000 m and
+    (2000 - lcl) / 1000 between; t_cin = 1 above -50 J/kg of mixed-layer CIN, 0 below -200 and (cin + 200) / 150 between
+    (``xp_supercell_tornado_parameters``, pointwise; NaN in gives NaN out)."""
+    return _pointwise("significant_tornado_parameter", [mlcape, effective_srh, effective_bulk_wind_difference,
+                                                        lcl_height, mlcin],
+                      name="significant_tornado_parameter", attrs=_ATTRS["significant_tornado_parameter"],
+                      device=device)
+
+
+def effective_layer_parameters(pressure, temperature, dewpoint, height, wind_u, wind_v, surface_wind_u,
+                               surface_wind_v, mover="right", min_cape=100, min_cin=-250, most_unstable_depth=300,
+                               mixed_layer_depth=100, vert_dim="model_level_number", vert_axis=0, device=None,
+                               **kwargs):
+    """Effective storm-relative helicity (ESRH), effective bulk wind difference (EBWD), the supercell composite
+    parameter and the effective-layer significant tornado parameter (contract in DESIGN.md section 3.14).
+
+    The effective inflow layer is ``effective_inflow_layer``'s (``min_cape``, ``min_cin``, ``most_unstable_depth`` and
+    ``kwargs``, cape_cin's options); one lift gives the mixed-layer (``mixed_layer_depth`` hPa) and most-unstable
+    (``most_unstable_depth`` hPa) parcels.  ``height`` is m above the surface on the levels of ``pressure``; the
+    heights of the layer's base and top, the MU equilibrium level and the ML LCL are ``log_interp`` of it.  ESRH is
+    the SRH of the ``mover``'s Bunkers motion over the layer; EBWD is the bulk wind difference from the base (at least
+    the surface) up to half the MU EL height above it.  Columns without an effective layer have NaN ESRH and EBWD and
+    enter the composites with ESRH = EBWD = 0 (so SCP and STP are 0 there unless another input is NaN); for
+    ``mover='left'`` the composites take -ESRH.  Returns a Dataset of effective_inflow_base / _top [hPa],
+    effective_srh [m2/s2], effective_bulk_wind_difference [m/s], supercell_composite_parameter and
+    significant_tornado_parameter."""
+    lookup_tables_loaded(device)
+    ctx = _lib.get_context(device)
+    lay, dtype, on_gpu = _layout_of(temperature, vert_dim, vert_axis)
+    dev = f"cuda:{ctx.device}"
+    t, td, p = [b.to(dev).contiguous() for b in _blocks(lay, [temperature, dewpoint, pressure], dtype)]
+    u, v, h = [b.to(dev) for b in _blocks(lay, [wind_u, wind_v, height], dtype)]
+    su, sv = [lay.scalar_to_block(x, dtype).to(dev) for x in (surface_wind_u, surface_wind_v)]
+    opt = _options(kwargs)
+    _clear_flags(ctx)
+    eff = ctx.effective_inflow_layer(p, t, td, options=_lib.make_options(most_unstable_depth=most_unstable_depth, **opt),
+                                     min_cape=min_cape, min_cin=min_cin)
+    lifted = ctx.cape_cin(p, t, td, kinds=("ml", "mu"), options=_lib.make_options(
+        mixed_layer_depth=mixed_layer_depth, most_unstable_depth=most_unstable_depth, **opt))
+    _check_flags(ctx)
+    base, top = eff["effective_inflow_base"], eff["effective_inflow_top"]
+    ml, mu = lifted["ml"], lifted["mu"]
+    hc = h.contiguous()
+    (z_base,), (z_top,), (z_el,), (z_lcl,) = [ctx.interp_levels(p, [hc], x, log=True)
+                                              for x in (base, top, mu["el_pressure"], ml["lcl_pressure"])]
+    zb0 = torch.clamp(z_base, min=0.0)                               # NaN stays NaN, like np.maximum
+    kin = ctx.storm_kinematics(h, u, v, su, sv, mover=mover, srh_layer=(z_base, z_top),
+                               bwd_layer=(zb0, zb0 + (z_el - zb0) / 2.0),
+                               outputs=["srh_layer", "bulk_wind_difference"])
+    no_layer = torch.isnan(base)
+    esrh = torch.where(no_layer, torch.full_like(base, float("nan")), kin["srh_layer"])
+    ebwd = torch.where(no_layer, torch.full_like(base, float("nan")), kin["bulk_wind_difference"])
+    s_in = torch.where(no_layer, torch.zeros_like(esrh), esrh) * _lib.MOVERS[mover]
+    b_in = torch.where(no_layer, torch.zeros_like(ebwd), ebwd)
+    comp = ctx.supercell_tornado_parameters(mu["cape"], s_in, b_in, ml["cape"], ml["cin"], z_lcl)
+    fix = (lambda x: x) if on_gpu else (lambda x: x.cpu())
+    out = {"effective_inflow_base": base, "effective_inflow_top": top, "effective_srh": esrh,
+           "effective_bulk_wind_difference": ebwd}
+    out.update(comp)
+    return lay.dataset({k: lay.wrap_scalar(fix(x), k) for k, x in out.items()})
+
+
 def _vertical_pressure(pressure, lay):
     """A shared 1-D pressure axis [L] reshaped to broadcast along the layout's vertical axis.  The pointwise functions
     broadcast like NumPy, which would align [L] with the last axis of the fields instead; anything else (per-point
@@ -1204,7 +1341,8 @@ def storm_proxies(dat, device=None):
     return ds
 
 
-def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat, downdraft=False, effective=False):
+def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat, downdraft=False, effective=False,
+          kinematics=False, mover="right"):
     p, t = dat["pressure"], dat["temperature"]
     td = dewpoint_from_specific_humidity(_vertical_pressure(p, _Layout(t, vert_dim, vert_axis)), t,
                                          dat["specific_humidity"], metpy_compat, device=device)
@@ -1249,7 +1387,14 @@ def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat, 
                      dat["wind_height_above_surface"], shear_height=6000, **kw))
     if downdraft:
         out["dcape"] = downdraft_cape(p, t, td, metpy_compat=metpy_compat, **kw)["dcape"]
-    if effective:
+    winds = (dat["surface_wind_u"], dat["surface_wind_v"], dat["wind_u"], dat["wind_v"], dat["wind_height_above_surface"])
+    if kinematics:
+        merge(bunkers_storm_motion(*winds, **kw))
+        merge(storm_relative_helicity(*winds, depths=(1000, 3000), mover=mover, **kw))
+    if effective and kinematics:
+        merge(effective_layer_parameters(p, t, td, winds[4], winds[2], winds[3], winds[0], winds[1], mover=mover,
+                                         metpy_compat=metpy_compat, **kw))
+    elif effective:
         eff = effective_inflow_layer(p, t, td, metpy_compat=metpy_compat, **kw)
         for k in _lib.EFFECTIVE_FIELDS:
             out[k] = eff[k]
@@ -1280,15 +1425,21 @@ def _conv(dat, vert_dim, vert_axis, device, min_set, ignore_nans, metpy_compat, 
 
 
 def conv_properties(dat, vert_dim="model_level_number", ignore_nans=False, vert_axis=0, device=None,
-                    metpy_compat="1.4.1", downdraft=False, effective=False):
+                    metpy_compat="1.4.1", downdraft=False, effective=False, kinematics=False, mover="right"):
     """PF:1951-2100: MU (250 hPa) and mixed (100, 50 hPa) CAPE/CIN, lifted and deep-convective indices,
     MU mixing ratio, 700-500 hPa lapse rate, 500 hPa temperature, freezing/melting level, 0-6 km shear.
     ``dat``: Dataset/dict with pressure, temperature, specific_humidity, height_asl, wind_u, wind_v,
     wind_height_above_surface (all [level, ...]) and surface_wind_u, surface_wind_v.  ``downdraft=True`` adds
     ``dcape`` (``downdraft_cape`` on the dewpoint derived from the specific humidity), masked like the rest;
     ``effective=True`` adds ``effective_inflow_base`` and ``effective_inflow_top`` (``effective_inflow_layer`` with
-    its defaults on that dewpoint), masked the same way."""
-    return _conv(dat, vert_dim, vert_axis, device, False, ignore_nans, metpy_compat, downdraft, effective)
+    its defaults on that dewpoint), masked the same way.  ``kinematics=True`` adds the Bunkers storm motion
+    (``bunkers_storm_motion``: bunkers_right_u/_v, bunkers_left_u/_v, mean_wind_u/_v) and srh_0_1000m / srh_0_3000m
+    (``storm_relative_helicity`` for ``mover``) on wind_height_above_surface and the surface wind; with
+    ``effective=True`` as well it adds effective_srh, effective_bulk_wind_difference, supercell_composite_parameter and
+    significant_tornado_parameter from one ``effective_layer_parameters`` call, whose base and top are the
+    effective_inflow_base / _top it returns.  All are masked like the rest."""
+    return _conv(dat, vert_dim, vert_axis, device, False, ignore_nans, metpy_compat, downdraft, effective, kinematics,
+                 mover)
 
 
 def min_conv_properties(dat, vert_dim="model_level_number", vert_axis=0, device=None, metpy_compat="1.4.1"):
