@@ -188,14 +188,17 @@ def effective_layer_parameters(pressure, temperature, dewpoint, height, wind_u, 
                                surface_wind_v, opts, mover=1, min_cape=100.0, min_cin=-250.0,
                                most_unstable_depth=300.0, mixed_layer_depth=100.0, pieces=None, **kwargs):
     """The effective-layer composition.  ``pieces``: the base / top pressures and the lift values (``lifts``'s keys
-    plus effective_inflow_base / _top) to compose from instead of computing them here.  Returns (outputs, scales)."""
+    plus effective_inflow_base / _top) to compose from instead of computing them here.  Returns (outputs, scales,
+    the pieces with the heights z_base, z_top, z_el, z_lcl; computed here, the pieces include the effective layer's
+    level_parcel_cape / _cin)."""
     t = np.asarray(temperature, np.float64)
     L, N = t.shape
     p = np.array(np.broadcast_to(op._as2d(pressure), (L, N)))
     if pieces is None:
         eff = eo.effective_inflow_layer(p, t, dewpoint, opts, min_cape, min_cin, most_unstable_depth, **kwargs)
         pieces = dict(lifts(p, t, dewpoint, opts, mixed_layer_depth, most_unstable_depth, **kwargs),
-                      effective_inflow_base=eff["effective_inflow_base"], effective_inflow_top=eff["effective_inflow_top"])
+                      **{k: eff[k] for k in ("effective_inflow_base", "effective_inflow_top", "level_parcel_cape",
+                                             "level_parcel_cin")})
     h = np.asarray(height, np.float64)
 
     def z_at(pr):
