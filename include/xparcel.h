@@ -174,7 +174,11 @@ xp_status xp_suite(xp_context *ctx, const xp_columns *cols, const xp_options *op
                    const xp_parcel_out *out_sb, const xp_parcel_out *out_ml,
                    const xp_parcel_out *out_mu, void *stream);
 
-/* ---- individually exposed steps (device memory only) ------------------------------------ */
+/* ---- individually exposed steps (device memory only) ------------------------------------
+ * These entries and the level / layer primitives below return XP_OK without a launch for n_columns = 0 and
+ * XP_ERR_INVALID_ARGUMENT for n_levels < 1, n_columns < 0 or, when more than one level is read or written, a level
+ * stride smaller than n_columns (the 1-D coordinate strides of a `*_is_1d` axis excepted): such a stride would let
+ * neighbouring columns read or write each other's elements. */
 /* lcl PF:609-682: [n] parcels -> lcl pressure/temperature/virtual temperature. */
 xp_status xp_lcl(xp_context *ctx, const void *parcel_pressure, const void *parcel_temperature,
                  const void *parcel_dewpoint, int64_t n, int32_t dtype, const xp_options *opts,

@@ -728,8 +728,11 @@ xp_status xp_moist_lapse(xp_context *ctx, const void *pressure, int64_t level_st
     if (!ctx) return XP_ERR_INVALID_ARGUMENT;
     std::lock_guard<std::mutex> lock(ctx->mu);
     if (!ctx->tables) return fail(ctx, XP_ERR_TABLES_NOT_LOADED, "Call load_moist_adiabat_lookups first.");
-    if (!pressure || !parcel_temperature || !parcel_pressure || !out_temperature)
+    if (n_columns == 0) return XP_OK;
+    if (!pressure || !parcel_temperature || !parcel_pressure || !out_temperature || n_levels < 1 || n_columns < 0)
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad moist_lapse arguments");
+    if (n_levels > 1 && (level_stride < n_columns || out_level_stride < n_columns))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "moist_lapse: level strides smaller than a level");
     DeviceGuard guard(ctx->device);
     Tables tb = {ctx->d_index, ctx->d_curves};
     cudaStream_t st = (cudaStream_t)stream;
@@ -749,8 +752,13 @@ xp_status xp_parcel_profile(xp_context *ctx, const void *pressure, int64_t level
     if (!ctx) return XP_ERR_INVALID_ARGUMENT;
     std::lock_guard<std::mutex> lock(ctx->mu);
     if (!ctx->tables) return fail(ctx, XP_ERR_TABLES_NOT_LOADED, "Call load_moist_adiabat_lookups first.");
-    if (!pressure || !parcel || !parcel->pressure || !parcel->temperature || !parcel->dewpoint)
+    if (n_columns == 0) return XP_OK;
+    if (!pressure || !parcel || !parcel->pressure || !parcel->temperature || !parcel->dewpoint || n_levels < 1 ||
+        n_columns < 0)
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad parcel_profile arguments");
+    if (n_levels > 1 && (level_stride < n_columns || ((out_temperature || out_virtual_temperature) &&
+                                                      out_level_stride < n_columns)))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "parcel_profile: level strides smaller than a level");
     DeviceGuard guard(ctx->device);
     Tables tb = {ctx->d_index, ctx->d_curves};
     const Opts o = to_opts(ctx, opts);
@@ -775,8 +783,12 @@ xp_status xp_lfc_el(xp_context *ctx, const void *pressure, const void *parcel_te
                     void *el_pressure, void *el_temperature, void *stream) {
     if (!ctx) return XP_ERR_INVALID_ARGUMENT;
     std::lock_guard<std::mutex> lock(ctx->mu);
-    if (!pressure || !parcel_temperature || !temperature || !lcl_pressure || !lcl_temperature)
+    if (n_columns == 0) return XP_OK;
+    if (!pressure || !parcel_temperature || !temperature || !lcl_pressure || !lcl_temperature || n_levels < 1 ||
+        n_columns < 0)
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad lfc_el arguments");
+    if (n_levels > 1 && level_stride < n_columns)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "lfc_el: level stride smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     XP_DISPATCH(dtype,
@@ -793,8 +805,12 @@ xp_status xp_cape_cin_base(xp_context *ctx, const void *pressure, const void *te
                            const xp_options *opts, void *cape, void *cin, void *stream) {
     if (!ctx) return XP_ERR_INVALID_ARGUMENT;
     std::lock_guard<std::mutex> lock(ctx->mu);
-    if (!pressure || !temperature || !parcel_temperature || !lfc_pressure || !el_pressure)
+    if (n_columns == 0) return XP_OK;
+    if (!pressure || !temperature || !parcel_temperature || !lfc_pressure || !el_pressure || n_levels < 1 ||
+        n_columns < 0)
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad cape_cin_base arguments");
+    if (n_levels > 1 && level_stride < n_columns)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "cape_cin_base: level stride smaller than a level");
     DeviceGuard guard(ctx->device);
     const Opts o = to_opts(ctx, opts);
     cudaStream_t st = (cudaStream_t)stream;
@@ -817,6 +833,8 @@ xp_status xp_interp_levels(xp_context *ctx, const void *coords, int64_t coords_l
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad interp_levels arguments");
     for (int f = 0; f < n_fields; ++f)
         if (!fields[f] || !outputs[f]) return fail(ctx, XP_ERR_INVALID_ARGUMENT, "interp_levels: NULL field/output");
+    if (n_levels > 1 && (level_stride < n_columns || (!coords_is_1d && coords_level_stride < n_columns)))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "interp_levels: level strides smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     XP_DISPATCH(dtype,
@@ -835,6 +853,8 @@ xp_status xp_level_crossing(xp_context *ctx, const void *coords, int64_t coords_
     if (n_columns == 0) return XP_OK;
     if (!coords || !field || !output || n_levels < 1 || n_columns < 0)
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad level_crossing arguments");
+    if (n_levels > 1 && (level_stride < n_columns || (!coords_is_1d && coords_level_stride < n_columns)))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "level_crossing: level strides smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     XP_DISPATCH(dtype,
@@ -856,6 +876,8 @@ xp_status xp_mixed_layer(xp_context *ctx, const void *pressure, int64_t pressure
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad mixed_layer arguments");
     for (int f = 0; f < n_fields; ++f)
         if (!fields[f] || !outputs[f]) return fail(ctx, XP_ERR_INVALID_ARGUMENT, "mixed_layer: NULL field/output");
+    if (n_levels > 1 && (level_stride < n_columns || (!pressure_is_1d && pressure_level_stride < n_columns)))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "mixed_layer: level strides smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     XP_DISPATCH(dtype,
@@ -874,6 +896,8 @@ xp_status xp_mixed_parcel(xp_context *ctx, const void *pressure, int64_t pressur
     if (n_columns == 0) return XP_OK;
     if (!pressure || !temperature || !dewpoint || !out || n_levels < 1 || n_columns < 0)
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad mixed_parcel arguments");
+    if (n_levels > 1 && (level_stride < n_columns || (!pressure_is_1d && pressure_level_stride < n_columns)))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "mixed_parcel: level strides smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     void *o6[6] = {out->theta, out->mixing_ratio, out->temperature, out->vapour_pressure, out->dewpoint, out->pressure};
@@ -892,6 +916,8 @@ xp_status xp_layer_bounds(xp_context *ctx, const void *pressure, int64_t pressur
     if (n_columns == 0) return XP_OK;
     if (!pressure || (!bottom_pressure && !top_pressure) || n_levels < 1 || n_columns < 0)
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad layer_bounds arguments");
+    if (n_levels > 1 && !pressure_is_1d && pressure_level_stride < n_columns)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "layer_bounds: level stride smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     XP_DISPATCH(dtype,
@@ -914,6 +940,10 @@ xp_status xp_insert_level(xp_context *ctx, const void *coords, int64_t coords_le
     for (int f = 0; f < n_fields; ++f)
         if (!fields[f] || !level_values[f] || !outputs[f])
             return fail(ctx, XP_ERR_INVALID_ARGUMENT, "insert_level: NULL field/level/output");
+    // the output always has n_levels + 1 >= 2 levels, so its stride is checked whatever n_levels is
+    if (out_level_stride < n_columns || (n_levels > 1 && ((n_fields > 0 && level_stride < n_columns) ||
+                                                          (!coords_is_1d && coords_level_stride < n_columns))))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "insert_level: level strides smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     XP_DISPATCH(dtype,
@@ -935,6 +965,8 @@ xp_status xp_shift_out_nans(xp_context *ctx, const void *ref_field, const void *
     for (int f = 0; f < n_fields; ++f)
         if (!fields[f] || !outputs[f] || fields[f] == outputs[f])
             return fail(ctx, XP_ERR_INVALID_ARGUMENT, "shift_out_nans: NULL or aliased field/output");
+    if (n_levels > 1 && level_stride < n_columns)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "shift_out_nans: level stride smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     XP_DISPATCH(dtype,
@@ -954,6 +986,9 @@ xp_status xp_trapz(xp_context *ctx, const void *x, int64_t x_level_stride, int32
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad trapz arguments");
     for (int f = 0; f < n_fields; ++f)
         if (!fields[f] || !outputs[f]) return fail(ctx, XP_ERR_INVALID_ARGUMENT, "trapz: NULL field/output");
+    if (n_levels > 1 && (level_stride < n_columns || (!x_is_1d && x_level_stride < n_columns) ||
+                         (mask && mask_level_stride < n_columns)))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "trapz: level strides smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     XP_DISPATCH(dtype,
@@ -972,6 +1007,9 @@ xp_status xp_find_intersections(xp_context *ctx, const void *x, int64_t x_level_
     if (n_columns == 0) return XP_OK;
     if (!x || !a || !b || !out || n_levels < 1 || n_columns < 0)
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad find_intersections arguments");
+    if (n_levels > 1 && (level_stride < n_columns || out_level_stride < n_columns ||
+                         (!x_is_1d && x_level_stride < n_columns)))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "find_intersections: level strides smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     void *o6[6] = {out->all_intersect_x, out->all_intersect_y, out->increasing_x, out->increasing_y,
@@ -1007,6 +1045,10 @@ xp_status xp_trap_around_zeros(xp_context *ctx, const void *x, int64_t x_level_s
     if (n_columns == 0) return XP_OK;
     if (!x || !y || !out || n_levels < 1 || n_columns < 0)
         return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad trap_around_zeros arguments");
+    // the area outputs have 2 n_levels - 1 levels: their stride matters from n_levels = 2 on, like the inputs'
+    if (n_levels > 1 && (level_stride < n_columns || out_level_stride < n_columns ||
+                         (!x_is_1d && x_level_stride < n_columns)))
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "trap_around_zeros: level strides smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     void *o5[5] = {out->area, out->x, out->dx, out->x_from, out->x_to};
@@ -1023,6 +1065,8 @@ xp_status xp_valid_data(xp_context *ctx, const void *pressure, int64_t pressure_
     std::lock_guard<std::mutex> lock(ctx->mu);
     if (n_columns == 0) return XP_OK;
     if (!pressure || n_levels < 1 || n_columns < 0) return fail(ctx, XP_ERR_INVALID_ARGUMENT, "bad valid_data arguments");
+    if (n_levels > 1 && !pressure_is_1d && pressure_level_stride < n_columns)
+        return fail(ctx, XP_ERR_INVALID_ARGUMENT, "valid_data: level stride smaller than a level");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t n = pressure_is_1d ? 1 : n_columns;

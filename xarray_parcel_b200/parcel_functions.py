@@ -449,6 +449,12 @@ def _names(dat):
     return list(dat.data_vars) if hasattr(dat, "data_vars") else list(dat.keys())
 
 
+def _template(arrays):
+    """The array whose shape is the columns' shape: the first of ``arrays`` with more than one dimension, so that a
+    shared 1-D pressure axis next to [L, N] fields lays out as the fields do (else the first array)."""
+    return next((a for a in arrays if getattr(a, "ndim", 0) > 1), arrays[0])
+
+
 def _full_blocks(lay, blocks):
     n = int(np.prod(lay.col_shape)) if lay.col_shape else 1
     return [b if b.dim() == 2 else b[:, None].expand(lay.L, n).contiguous() for b in blocks]
@@ -460,8 +466,8 @@ def insert_level(d, level, coords, vert_dim="model_level_number", fill_value=-99
     assert fill_value == -999, "only the reference's default fill_value is implemented"
     keys = _names(level)
     ctx = _lib.get_context(device)
-    lay, dtype, on_gpu = _layout_of(d[coords], vert_dim, vert_axis)
     others = [k for k in keys if k != coords]
+    lay, dtype, on_gpu = _layout_of(_template([d[coords]] + [d[k] for k in others]), vert_dim, vert_axis)
     blocks = _full_blocks(lay, _blocks(lay, [d[coords]] + [d[k] for k in others], dtype))
     lev = [lay.scalar_to_block(level[k], dtype).cuda().contiguous() for k in [coords] + others]
     assert not bool((blocks[0] == fill_value).any()), "dataset d contains fill_value."          # PF:962
@@ -511,7 +517,7 @@ def shift_out_nans(x, name, dim="model_level_number", vert_axis=0, device=None):
     """PF:1699-1720: shift every variable of ``x`` down, column by column, until level 0 of ``name`` is not NaN."""
     names = _names(x)
     ctx = _lib.get_context(device)
-    lay, dtype, on_gpu = _layout_of(x[name], dim, vert_axis)
+    lay, dtype, on_gpu = _layout_of(_template([x[name]] + [x[k] for k in names]), dim, vert_axis)
     blocks = _full_blocks(lay, _blocks(lay, [x[k] for k in names], dtype))
     outs, _ = ctx.shift_out_nans(blocks[names.index(name)], blocks)
     return lay.dataset({k: lay.wrap_profile(o if on_gpu else o.cpu(), k, lay.L) for k, o in zip(names, outs)})
@@ -577,7 +583,8 @@ def interp1d_numba(at, xp, fp, device=None):
     ctx = _lib.get_context(device)
     on_gpu = isinstance(fp, torch.Tensor) and fp.is_cuda
     is_t = isinstance(fp, torch.Tensor)
-    conv = lambda a: (a if isinstance(a, torch.Tensor) else torch.as_tensor(np.asarray(a, dtype=np.float64))).cuda()
+    dt = _float_dtype([fp])
+    conv = lambda a: (a if isinstance(a, torch.Tensor) else torch.as_tensor(np.asarray(a))).to(dt).cuda()  # noqa: E731
     out = ctx.interp1d(conv(at), conv(xp), conv(fp))
     return out if on_gpu else (out.cpu() if is_t else out.cpu().numpy())
 
@@ -604,7 +611,7 @@ def get_layer(dat, depth=100, vert_dim="model_level_number", interpolate=True, v
     level closest to it (bound_pressure)."""
     names = _names(dat)
     ctx = _lib.get_context(device)
-    lay, dtype, on_gpu = _layout_of(dat["pressure"], vert_dim, vert_axis)
+    lay, dtype, on_gpu = _layout_of(_template([dat["pressure"]] + [dat[k] for k in names]), vert_dim, vert_axis)
     blocks = _full_blocks(lay, _blocks(lay, [dat[k] for k in names], dtype))
     pb = blocks[names.index("pressure")]
     n = pb.shape[1]
@@ -760,6 +767,18 @@ def _back(t, template):
     return t.cpu().numpy()
 
 
+def _float_dtype(args):
+    """The dtype of a step's computation: that of the first float32 / float64 tensor or float32 NumPy array among
+    ``args`` (NumPy float64, Python scalars and other types compute in float64)."""
+    for a in args:
+        a = a.data if (_xr is not None and isinstance(a, _xr.DataArray)) else a
+        if isinstance(a, torch.Tensor) and a.dtype in (torch.float32, torch.float64):
+            return a.dtype
+        if isinstance(a, np.ndarray) and a.dtype == np.float32:
+            return torch.float32
+    return torch.float64
+
+
 def _pointwise(method, args, template=0, name=None, attrs=None, device=None, **kw):
     """Run a pointwise Context method (``_lib.Context.<method>``: one CUDA thread per point) on broadcast
     inputs and hand the result back as the template's array type (DataArray / torch / NumPy)."""
@@ -769,15 +788,8 @@ def _pointwise(method, args, template=0, name=None, attrs=None, device=None, **k
         xa = _xr.broadcast(*[a if isinstance(a, _xr.DataArray) else _xr.DataArray(a) for a in args])
         tmpl = xa[template]
         args = [a.data for a in xa]
-    dt = None
-    for a in args:
-        if isinstance(a, torch.Tensor) and a.dtype in (torch.float32, torch.float64):
-            dt = a.dtype
-            break
-        if isinstance(a, np.ndarray) and a.dtype == np.float32:
-            dt = torch.float32
-            break
-    dev = [_to_dev(a, dtype=dt or torch.float64) for a in args]
+    dt = _float_dtype(args)
+    dev = [_to_dev(a, dtype=dt) for a in args]
     res = getattr(ctx, method)(*dev, **kw)
     if _xr is not None and isinstance(tmpl, _xr.DataArray):
         out = tmpl.copy(data=res.cpu().numpy())
@@ -794,9 +806,8 @@ def _pointwise(method, args, template=0, name=None, attrs=None, device=None, **k
 def lcl(parcel_pressure, parcel_temperature, parcel_dewpoint, device=None, **kwargs):
     """PF:609-682.  Returns Dataset{lcl_pressure, lcl_temperature, lcl_virtual_temperature}."""
     ctx = _lib.get_context(device)
-    pt = _to_dev(parcel_temperature)
-    pp = _to_dev(parcel_pressure, dtype=pt.dtype)
-    pd = _to_dev(parcel_dewpoint, dtype=pt.dtype)
+    dt = _float_dtype([parcel_temperature, parcel_pressure, parcel_dewpoint])
+    pt, pp, pd = [_to_dev(x, dtype=dt) for x in (parcel_temperature, parcel_pressure, parcel_dewpoint)]
     a, b, c = ctx.lcl(pp, pt, pd, _lib.make_options(**_options(kwargs)))
     ds = Dataset({"lcl_pressure": _back(a, parcel_temperature), "lcl_temperature": _back(b, parcel_temperature),
                   "lcl_virtual_temperature": _back(c, parcel_temperature)})
@@ -832,18 +843,52 @@ def mixing_ratio(temperature, dewpoint, pressure, metpy_compat="1.4.1", device=N
                       metpy_compat=metpy_compat)
 
 
+def _lift_layout(pressure, parcels, vert_dim, vert_axis):
+    """Layout of a lift of ``parcels`` over ``pressure``.  A shared 1-D pressure axis under parcels of more than one
+    element takes its columns from the parcels: the profiles come back with the vertical dimension first, then the
+    parcels' dimensions, as if the axis had been broadcast against them."""
+    lay = _Layout(pressure, vert_dim, vert_axis)
+    if len(lay.shape) != 1:
+        return lay
+    raw_of = lambda x: x.data if (_xr is not None and isinstance(x, _xr.DataArray)) else x     # noqa: E731
+    shape_of = lambda x: tuple(x.shape) if isinstance(x, torch.Tensor) else np.shape(x)      # noqa: E731
+    par = next((x for x in parcels if x is not None and int(np.prod(shape_of(raw_of(x)))) > 1), None)
+    if par is None:
+        return lay
+    if lay.is_xr and isinstance(par, _xr.DataArray):
+        tmpl = _xr.broadcast(pressure, par)[0]
+        tmpl = tmpl.transpose(vert_dim, *[d for d in tmpl.dims if d != vert_dim])
+        return _Layout(tmpl, vert_dim, 0)
+    shape = shape_of(raw_of(par))
+    raw = pressure.data if lay.is_xr else pressure
+    lead = (slice(None),) + (None,) * len(shape)
+    if isinstance(raw, torch.Tensor):
+        tmpl = raw[lead].expand(raw.shape[0], *shape)
+    else:
+        raw = np.asarray(raw)
+        tmpl = np.broadcast_to(raw[lead], raw.shape + shape)
+    return _Layout(tmpl, vert_dim, 0)
+
+
+def _lift_pressure(lay, pressure, dtype):
+    """Pressure of a lift as a contiguous CUDA block [L, N] (a shared axis broadcast over the layout's columns)."""
+    p = lay.to_block(pressure, None, dtype).cuda()
+    if p.dim() == 1:
+        n = int(np.prod(lay.col_shape)) if lay.col_shape else 1
+        p = p[:, None].expand(p.shape[0], n)
+    return p.contiguous()
+
+
 def moist_lapse(pressure, parcel_temperature, parcel_pressure=None, vert_dim="model_level_number",
                 persist=True, vert_axis=0, device=None):
     """PF:525-607: lookup-table moist adiabat.  ``pressure`` is [L, ...] (vertical axis first for
     plain arrays)."""
     ctx = _lib.get_context(device)
     lookup_tables_loaded(device)
-    lay = _Layout(pressure, vert_dim, vert_axis)
+    lay = _lift_layout(pressure, (parcel_temperature, parcel_pressure), vert_dim, vert_axis)
     raw = pressure.data if lay.is_xr else pressure
     dtype = raw.dtype if isinstance(raw, torch.Tensor) else (torch.float32 if np.asarray(raw).dtype == np.float32 else torch.float64)
-    p = lay.to_block(pressure, None, dtype).cuda()
-    if p.dim() == 1:
-        p = p[:, None]
+    p = _lift_pressure(lay, pressure, dtype)
     if parcel_pressure is None:
         parcel_pressure = p[0]
         pp = parcel_pressure
@@ -860,13 +905,11 @@ def parcel_profile(pressure, parcel_pressure, parcel_temperature, parcel_dewpoin
     """PF:712-780: parcel temperature / virtual temperature on the input levels + the LCL."""
     ctx = _lib.get_context(device)
     lookup_tables_loaded(device)
-    lay = _Layout(pressure, vert_dim, vert_axis)
+    lay = _lift_layout(pressure, (parcel_pressure, parcel_temperature, parcel_dewpoint), vert_dim, vert_axis)
     raw = pressure.data if lay.is_xr else pressure
     dtype = raw.dtype if isinstance(raw, torch.Tensor) else (torch.float32 if np.asarray(raw).dtype == np.float32 else torch.float64)
     on_gpu = isinstance(raw, torch.Tensor) and raw.is_cuda
-    p = lay.to_block(pressure, None, dtype).cuda()
-    if p.dim() == 1:
-        p = p[:, None]
+    p = _lift_pressure(lay, pressure, dtype)
     pp = lay.scalar_to_block(parcel_pressure, dtype).cuda()
     pt = lay.scalar_to_block(parcel_temperature, dtype).cuda()
     pd = lay.scalar_to_block(parcel_dewpoint, dtype).cuda()
@@ -896,6 +939,7 @@ def lfc_el(pressure, parcel_temperature, temperature, lcl_pressure, lcl_temperat
         blocks.append(b.contiguous())
     lp = lay.scalar_to_block(lcl_pressure, dtype).cuda()
     lt = lay.scalar_to_block(lcl_temperature, dtype).cuda()
+    _clear_flags(ctx)
     r = ctx.lfc_el(blocks[0], blocks[1], blocks[2], lp, lt)
     _check_flags(ctx)
     fix = (lambda x: x) if on_gpu else (lambda x: x.cpu())
